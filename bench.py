@@ -3,6 +3,7 @@
 at global batch 32768 x 128-d, tau = 0.5, normalize = True, on 1/2/4/8 B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA path
+    python bench.py --dump-outputs DIR [...]                        # ... and write its last step's outputs to DIR
     python bench.py --impl reference [...]                          # CPU arm (oracle port, host cores)
     torchrun --nproc-per-node N bench.py --gpus N ...               # N > 1: one rank per GPU, NCCL
 
@@ -287,6 +288,16 @@ def parity_witness(zi, zj, dzi, loss_value, world, rank, dist_mod, rows=4096, ta
                        "max over ranks"}
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy in float32, so that two builds run with the same arguments (hence the
+    same seeded inputs) can be compared output by output.  At one GPU that is the loss and both 32768 x 128 gradients:
+    32 MiB in all."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ----------------------------------------------------------------------------------------- GPU arm
 def run_ours(args):
     import torch
@@ -323,12 +334,14 @@ def run_ours(args):
     zj = h_zj.to(dev).requires_grad_(True)
     loss_fn = ssv_b200.SimclrLoss(True, TAU) if world == 1 else DistributedSimclrLoss(True, TAU)
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)  # > 126 MB L2
+    last = {}
 
     def step_resident():
         zi.grad = None
         zj.grad = None
         loss = loss_fn(zi, zj)
         loss.backward()
+        last["loss"] = loss
         return loss
 
     # e2e: what a training loop does — the next step's inputs travel host->device on a side stream (pinned memory,
@@ -406,7 +419,11 @@ def run_ours(args):
     sampler.mark()
     ms_step, launches, prof = timed(step_resident, args.steps, args.warmup, profile=True)
     clocks = sampler.stop()
+    # what the last timed step handed its caller; the steps below allocate fresh gradients and leave these untouched
+    outputs = {"loss": last["loss"], "dzi": zi.grad, "dzj": zj.grad}
     ms_e2e, _, _ = timed(step_e2e, args.steps, max(3, args.warmup // 2))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
 
     # correctness evidence carried by the bench line itself (every N): one more step, outside the timed regions
     zi.grad = None
@@ -496,7 +513,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--no-per-config", action="store_true", help="skip the per_config array (the other BASELINE configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss and the gradients of the last timed step (rank 0's "
+                         "rows) as DIR/loss.npy, DIR/dzi.npy, DIR/dzj.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

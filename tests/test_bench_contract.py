@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -36,6 +38,16 @@ def test_reference_arm_json_line():
 
 def test_reference_arm_other_ranks_exit_quietly():
     assert _run({"RANK": "3", "WORLD_SIZE": "8", "LOCAL_RANK": "3"}) == []
+
+
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "DIR"]])
+def test_bad_arguments_are_refused(tmp_path, extra):
+    """No timed step means no time, and --dump-outputs writes what the CUDA path returns, so both are usage errors."""
+    args = [a.replace("DIR", str(tmp_path / "out")) for a in extra]
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                         timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and "error:" in out.stderr
+    assert not (tmp_path / "out").exists()
 
 
 def test_reference_arm_falls_back_to_port_without_reference(tmp_path):
