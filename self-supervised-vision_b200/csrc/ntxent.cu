@@ -99,6 +99,14 @@ WsLayout ws_layout(void* base, int64_t local_rows, int64_t row_blocks, int64_t c
   p.cols = static_cast<int>(cols);
   plan_chunks(p, sim_fwd_bn(dpad), sim_fwd_min_tiles(dpad));
   size_t part_elems = static_cast<size_t>(4 * p.nchunks + 2) * lr;
+  if (local_rows == cols && dpad <= 128) {
+    // single GPU: the symmetric forward's row partials, then its (R - 1) / 2 column partials per row
+    SimParams q{};
+    q.row_blocks = static_cast<int>(row_blocks);
+    const int ncol = plan_sym(q);
+    const size_t sym_elems = static_cast<size_t>(4 * q.nchunks + ncol) * lr;
+    if (part_elems < sym_elems) part_elems = sym_elems;
+  }
   if (part_elems < static_cast<size_t>(sim_mpad(cols))) part_elems = sim_mpad(cols);
   w.pos = c.take<float>(lr);
   w.part_m = c.take<float>(part_elems);
@@ -227,24 +235,35 @@ int ssvb_ntxent_fwd(const float* zi, const float* zj, int64_t n, int64_t d, int6
   }
   SimParams p;
   fill_sim_params_rows(p, pl, 1, pl.m, 0, 0);
-  plan_chunks(p, sim_fwd_bn(pl.dpad), sim_fwd_min_tiles(pl.dpad));
   p.part_m = ws.part_m;
   p.part_l = ws.part_l;
   p.part_stride = static_cast<int>(round_up(pl.m, 256));
 #ifdef SSVB_DBG_TIMING
   if (const char* e = getenv("SSVB_DBG_PTR")) p.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
 #endif
-  SSVB_TRY(launch_sim_fwd(pl.mode, sv.zhat, pl.mpad, sv.zhat, pl.mpad, pl.dpad, p, s));
+  // FIXED mode needs no running max, so S = S^T is exploited: every tile is computed once and also yields the row
+  // sums of its mirror (column partials after the row partials, summed by the finalize in index order)
+  int nparts;
+  if (pl.mode == SIM_NTX_FIXED && pl.dpad <= 128) {
+    const int ncol = plan_sym(p);
+    p.colpart = ws.part_l + static_cast<size_t>(4 * p.nchunks) * p.part_stride;
+    nparts = 4 * p.nchunks + ncol;
+    SSVB_TRY(launch_sim_fwd_sym(sv.zhat, pl.mpad, pl.dpad, p, s));
+  } else {
+    plan_chunks(p, sim_fwd_bn(pl.dpad), sim_fwd_min_tiles(pl.dpad));
+    nparts = 4 * p.nchunks;
+    SSVB_TRY(launch_sim_fwd(pl.mode, sv.zhat, pl.mpad, sv.zhat, pl.mpad, pl.dpad, p, s));
+  }
   {
     const unsigned grid = static_cast<unsigned>(ceil_div(pl.m, 256));
     const float scale = 1.f / static_cast<float>(pl.m);
     if (pl.mode == SIM_NTX_FIXED)
-      lse_finalize_kernel<SIM_NTX_FIXED><<<grid, 256, 0, s>>>(ws.part_m, ws.part_l, 4 * p.nchunks, p.part_stride,
+      lse_finalize_kernel<SIM_NTX_FIXED><<<grid, 256, 0, s>>>(ws.part_m, ws.part_l, nparts, p.part_stride,
                                                             static_cast<int>(pl.m), ws.pos, pl.c, pl.shift,
                                                             sv.stat, nullptr, ws.block_sums, ws.counter, scale, loss,
                                                             nullptr, nullptr, 0, 0, pl.wscale);
     else
-      lse_finalize_kernel<SIM_NTX_ONLINE><<<grid, 256, 0, s>>>(ws.part_m, ws.part_l, 4 * p.nchunks, p.part_stride,
+      lse_finalize_kernel<SIM_NTX_ONLINE><<<grid, 256, 0, s>>>(ws.part_m, ws.part_l, nparts, p.part_stride,
                                                              static_cast<int>(pl.m), ws.pos, pl.c, pl.shift,
                                                              sv.stat, nullptr, ws.block_sums, ws.counter, scale, loss);
     SSVB_LAUNCH_CHECK();

@@ -17,8 +17,8 @@ inline int sim_fwd_min_tiles(int64_t dpad) { return 1024 / sim_fwd_bn(dpad); }
 // Choose the column chunking: (row block, chunk) units are statically strided over one CTA per SM, so the number
 // of units should fill whole waves of `num_sms()` CTAs (tail effect) while every chunk keeps >= min_tiles tiles
 // (amortises the A-tile load, the partial write / the accumulator drain).  No chunk is ever empty.
-inline void plan_chunks(SimParams& p, int BN, int min_tiles) {
-  p.col_tiles = static_cast<int>(ceil_div(p.cols, BN));
+inline void plan_chunks_tiles(SimParams& p, int col_tiles, int min_tiles) {
+  p.col_tiles = col_tiles;
   const int sms = num_sms();
   const int max_ch = p.col_tiles / min_tiles > 1 ? p.col_tiles / min_tiles : 1;
   int best = 1;
@@ -39,6 +39,38 @@ inline void plan_chunks(SimParams& p, int BN, int min_tiles) {
   }
   p.tiles_per_chunk = static_cast<int>(ceil_div(p.col_tiles, best));
   p.nchunks = static_cast<int>(ceil_div(p.col_tiles, p.tiles_per_chunk));
+}
+inline void plan_chunks(SimParams& p, int BN, int min_tiles) {
+  plan_chunks_tiles(p, static_cast<int>(ceil_div(p.cols, BN)), min_tiles);
+}
+// symmetric forward (sim_fwd_sym_kernel): p.row_blocks = R row blocks of a square S; each takes a band of
+// floor(R/2) + 1 128-column tiles, two per 256-column stage.  Returns the number of column partials per row
+// ((R - 1) / 2, stored after the 4 * nchunks row partials).
+inline int plan_sym(SimParams& p) {
+  p.band = p.row_blocks / 2 + 1;
+  plan_chunks_tiles(p, (p.band + 1) / 2, sim_fwd_min_tiles(128));
+  return (p.row_blocks - 1) / 2;
+}
+
+template <int KB>
+int launch_sim_fwd_sym_t(const CUtensorMap& tmA, const CUtensorMap& tmB, const SimParams& p, cudaStream_t s) {
+  auto kern = sim_fwd_sym_kernel<KB, true>;
+  constexpr int smem = SymCfg<KB>::SMEM;
+  SSVB_TRY((set_smem_once<sim_fwd_sym_kernel<KB, true>>(smem)));
+  const int nunits = p.row_blocks * p.nchunks;
+  const int grid = nunits < num_sms() ? nunits : num_sms();
+  const int slot = prof_begin(PROF_SIM_FWD, s);
+  kern<<<grid, 640, smem, s>>>(tmA, tmB, p);
+  prof_end(slot, s);
+  SSVB_LAUNCH_CHECK();
+  return SSVB_OK;
+}
+// Z: fp16 [z_rows x dpad] (unit-norm rows, pre-scaled; FIXED mode only), dpad <= 128
+inline int launch_sim_fwd_sym(const void* Z, int64_t z_rows, int64_t dpad, const SimParams& p, cudaStream_t s) {
+  if (!p.opf16 || dpad > 128) return SSVB_ERR_UNSUPPORTED;
+  CUtensorMap tm;  // A and B are the same matrix, both in 128-row boxes
+  SSVB_TRY(make_tmap_bf16(&tm, Z, z_rows, dpad, dpad, 128, true));
+  return dpad == 64 ? launch_sim_fwd_sym_t<1>(tm, tm, p, s) : launch_sim_fwd_sym_t<2>(tm, tm, p, s);
 }
 
 template <int KB, int MODE, bool OPF16 = false>

@@ -31,6 +31,9 @@ struct SimParams {
   float* part_m;
   float* part_l;
   int part_stride;
+  // symmetric forward (sim_fwd_sym_kernel): band tiles per row block, column partials [(R - 1) / 2][part_stride]
+  int band;
+  float* colpart;
   // backward inputs / outputs
   const float* rowstat;  // NT-Xent: indexed by global row; MoCo: by local row
   const float* colstat;  // NT-Xent: fp32 column statistic (FIXED: 1/L', ONLINE: lse2), padded to a multiple of 128
@@ -414,6 +417,308 @@ sim_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (p.dbg && blockIdx.x == 0 && warp == 4 && lane == 0)
       for (int i = 0; i < 8; ++i) p.dbg[16 + i] = static_cast<unsigned long long>(_t_acc[i]);
 #endif
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) tmem_dealloc<512>(tmem);
+}
+
+// =====================================================================================================
+// symmetric forward (single GPU, FIXED mode, dpad <= 128): S = Z Z^T, so each 128 x 128 tile is computed once
+// =====================================================================================================
+// Row block i (R = row_blocks) takes the cyclic band of column blocks b = (i + o) mod R, o = 0 .. floor(R/2)
+// (p.band = floor(R/2) + 1 tiles):
+//   o = 0          diagonal tile: row sums only, diagonal element masked;
+//   1 <= o < R/2   full tile: row sums -> block i, column sums -> block b (p.colpart[o - 1][b * 128 + col]);
+//   o = R/2        (R even) antipodal tile, reached from both partners: each takes row sums only.
+// So exp2(t_ab) enters L_a exactly once for every pair of valid rows a != b.  A 256-column stage holds the tiles
+// o = 2t and 2t + 1 (two 128-row TMA boxes, block coordinates taken mod R); when the band length is odd the second half
+// of the last stage is loaded and multiplied but not read.  Staged rows >= M are zero (logit 0, exp2 = 1): they are
+// masked out of both sums.
+//
+// Column sums: the softmax warps read S with tcgen05.ld.16x256b (the mma accumulator fragment: thread 4g + c holds
+// rows g, g + 8 (+16, +24 from the second load) and columns 8k + 2c, 8k + 2c + 1), so one thread covers 4 rows and the
+// rows of a column are spread over 8 lanes instead of 32.  Per pair of exponentials: one packed add into the row
+// accumulator and one into the column accumulator.  Each warp stores its per-lane column partials (8 floats per 32
+// columns) to shared memory; after a warpgroup barrier two warps sum the 32 partials of each column in a fixed order
+// and write one 128-float partial per tile (deterministic: no float atomics).
+template <int KB>
+struct SymCfg {
+  static constexpr int BN = 256;
+  static constexpr int A_BYTES = 128 * 128 * KB;
+  static constexpr int B_BYTES = BN * 128 * KB;
+  // d = 128: a 2-stage ring is what leaves room for the 64 KB of column-partial buffers in 227 KB
+  static constexpr int NSTAGE = (KB == 1) ? 4 : 2;
+  static constexpr int CP_BYTES = 4 * 16384;  // per softmax warpgroup: [chunk 4][warp 4][g 8][32 floats]
+  static constexpr int NBARS = 4 + 2 * NSTAGE + 4;
+  static constexpr int SMEM = 1024 + A_BYTES + NSTAGE * B_BYTES + CP_BYTES + NBARS * 8 + 16;
+};
+
+// TMEM -> registers, 16 lanes x 8 columns x 4 repetitions (see the layout note above)
+__device__ __forceinline__ void tmem_ld_16x256b_x4(uint32_t taddr, uint32_t* v) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.16x256b.x4.b32 "
+      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+        "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+      : "r"(taddr)
+      : "memory");
+}
+__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+
+// one 128 x 128 tile (this warp: 32 rows).  COLS: also store the column partials of each 32-column chunk to `cp`
+// (this warp's slot of the warpgroup buffer).  MASKED: diag = diagonal tile; rows / columns >= p.cols are padding.
+template <bool MASKED, bool COLS>
+__device__ __forceinline__ void sym_tile(uint32_t taddr, const SimParams& p, unsigned long long (&racc)[4],
+                                         uint32_t a_s_empty, int lane, uint32_t cp_st0, uint32_t cp_st1, int barid,
+                                         int row_w, int col_t, bool diag) {
+  uint32_t v[2][32];
+  tmem_ld_16x256b_x4(taddr, v[0]);
+  tmem_ld_16x256b_x4(taddr + (16u << 16), v[0] + 16);
+  const int g = lane >> 2, c4 = lane & 3;
+#pragma unroll
+  for (int cc = 0; cc < 4; ++cc) {
+    uint32_t(&cur)[32] = v[cc & 1];
+    tmem_ld_wait_regs(cur);
+    if (cc < 3) {
+      tmem_ld_16x256b_x4(taddr + (cc + 1) * 32, v[(cc + 1) & 1]);
+      tmem_ld_16x256b_x4(taddr + (16u << 16) + (cc + 1) * 32, v[(cc + 1) & 1] + 16);
+    } else {
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive_a(a_s_empty);
+    }
+    unsigned long long cacc[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {  // row slot r: row g + 8 r of this warp's 32
+        const int idx = 16 * (r >> 1) + 4 * k + 2 * (r & 1);
+        unsigned long long e2;
+        if (MASKED) {
+          const int row = row_w + g + 8 * r, col = col_t + cc * 32 + 8 * k + 2 * c4;
+          float e[2];
+#pragma unroll
+          for (int j = 0; j < 2; ++j) {
+            const bool off = (diag && row == col + j) || row >= p.cols || col + j >= p.cols;
+            e[j] = ex2f(off ? -INFINITY : __uint_as_float(cur[idx + j]));
+          }
+          e2 = pack_f32x2(e[0], e[1]);
+        } else if (((4 * k + r) % SSVB_POLY_FWD_MOD) < SSVB_POLY_FWD_CNT) {
+          e2 = ex2_poly3_x2(pack_f32x2(__uint_as_float(cur[idx]), __uint_as_float(cur[idx + 1])));
+        } else {
+          e2 = pack_f32x2(SSVB_EX2(__uint_as_float(cur[idx])), SSVB_EX2(__uint_as_float(cur[idx + 1])));
+        }
+        racc[r] = add_f32x2(racc[r], e2);
+        if (COLS) cacc[k] = r == 0 ? e2 : add_f32x2(cacc[k], e2);
+      }
+    }
+    if (COLS) {
+      // the two readers of the previous tile's partials are done before the first store of this tile
+      if (cc == 0) named_bar_sync(barid, 128);
+      const uint32_t o = cc * 4096;
+      asm volatile("st.shared.v2.b64 [%0], {%1, %2};" ::"r"(cp_st0 + o), "l"(cacc[0]), "l"(cacc[1]) : "memory");
+      asm volatile("st.shared.v2.b64 [%0], {%1, %2};" ::"r"(cp_st1 + o), "l"(cacc[2]), "l"(cacc[3]) : "memory");
+    }
+  }
+}
+
+template <int KB, bool OPF16>
+__global__ void __launch_bounds__(640, 1)
+sim_fwd_sym_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const SimParams p) {
+  using C = SymCfg<KB>;
+  constexpr int BN = C::BN, NSTAGE = C::NSTAGE, NBUF = 2;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = align1024(smem_raw);
+  uint8_t* sA = smem;
+  uint8_t* sB = smem + C::A_BYTES;
+  uint8_t* sCP = sB + NSTAGE * C::B_BYTES;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sCP + C::CP_BYTES);
+  uint64_t* a_full = bars;
+  uint64_t* a_empty = bars + 2;
+  uint64_t* b_full = bars + 4;
+  uint64_t* b_empty = b_full + NSTAGE;
+  uint64_t* s_full = b_empty + NSTAGE;
+  uint64_t* s_empty = s_full + NBUF;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(s_empty + NBUF);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int R = p.row_blocks;
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&tmA);
+    tma_prefetch_desc(&tmB);
+  }
+  if (warp == 1 && lane == 0) {
+    mbar_init(&a_full[0], 1);
+    mbar_init(&a_empty[0], 1);
+    for (int i = 0; i < NBUF; ++i) {
+      mbar_init(&s_full[i], 1);
+      mbar_init(&s_empty[i], 8);  // the warpgroup pair that drains the buffer
+    }
+    for (int i = 0; i < NSTAGE; ++i) {
+      mbar_init(&b_full[i], 1);
+      mbar_init(&b_empty[i], 1);
+    }
+    fence_barrier_init();
+  }
+  if (warp == 2) tmem_alloc<512>(tmem_slot);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tmem_slot;
+  const int nunits = p.row_blocks * p.nchunks;
+
+  if (warp < 4) {
+    asm volatile("setmaxnreg.dec.sync.aligned.u32 40;");
+    if (warp == 0) {
+      // ---------------------------------------------------------------- TMA producer
+      int ucount = 0, gt = 0;
+      for (int u = blockIdx.x; u < nunits; u += gridDim.x, ++ucount) {
+        const UnitInfo ui = decode_unit(p, u);
+        const int rb = ui.g0 >> 7;
+        mbar_wait(&a_empty[0], (ucount & 1) ^ 1);
+        if (elect_one()) {
+          mbar_expect_tx(&a_full[0], C::A_BYTES);
+#pragma unroll
+          for (int kb = 0; kb < KB; ++kb) tma_load_2d(sA + kb * (128 * 128), &tmA, &a_full[0], kb * 64, ui.g0);
+        }
+        __syncwarp();
+        for (int t = ui.t0; t < ui.t1; ++t, ++gt) {
+          const int st = gt % NSTAGE;
+          mbar_wait(&b_empty[st], ((gt / NSTAGE) & 1) ^ 1);
+          if (elect_one()) {
+            mbar_expect_tx(&b_full[st], C::B_BYTES);
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+              const int b = (rb + 2 * t + h) % R;
+#pragma unroll
+              for (int kb = 0; kb < KB; ++kb)
+                tma_load_2d(sB + st * C::B_BYTES + kb * (BN * 128) + h * (128 * 128), &tmB, &b_full[st], kb * 64,
+                            b * 128);
+            }
+          }
+          __syncwarp();
+        }
+      }
+    } else if (warp == 1) {
+      // ---------------------------------------------------------------- MMA issuer
+      constexpr uint32_t IDESC = make_idesc(128, BN, 0, 0, OPF16 ? 0 : 1);
+      const uint32_t abase = smem_u32(sA);
+      int ucount = 0, gt = 0;
+      for (int u = blockIdx.x; u < nunits; u += gridDim.x, ++ucount) {
+        const UnitInfo ui = decode_unit(p, u);
+        mbar_wait(&a_full[0], ucount & 1);
+        for (int t = ui.t0; t < ui.t1; ++t, ++gt) {
+          const int st = gt % NSTAGE, buf = gt % NBUF;
+          mbar_wait(&b_full[st], (gt / NSTAGE) & 1);
+          mbar_wait(&s_empty[buf], ((gt / NBUF) & 1) ^ 1);
+          tc_fence_after();
+          if (elect_one()) {
+            const uint32_t bbase = smem_u32(sB + st * C::B_BYTES);
+#pragma unroll
+            for (int kb = 0; kb < KB; ++kb)
+#pragma unroll
+              for (int k4 = 0; k4 < 4; ++k4)
+                umma_ss(tmem + buf * BN, desc_kmajor(abase + kb * (128 * 128) + k4 * 32),
+                        desc_kmajor(bbase + kb * (BN * 128) + k4 * 32), IDESC, (kb | k4) != 0);
+            umma_commit(&b_empty[st]);
+            umma_commit(&s_full[buf]);
+            if (t == ui.t1 - 1) umma_commit(&a_empty[0]);
+          }
+          __syncwarp();
+        }
+      }
+    }
+  } else {
+    // ------------------------------------------------------------------ softmax warpgroups
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 104;");
+    const int wgi = (warp - 4) >> 2;  // 0..3
+    const int pair = wgi >> 1, half = wgi & 1;
+    const int q = warp & 3;
+    const int g = lane >> 2, c4 = lane & 3;
+    const uint32_t tlane = static_cast<uint32_t>(q * 32) << 16;
+    const uint32_t a_s_full = smem_u32(&s_full[pair]), a_s_empty = smem_u32(&s_empty[pair]);
+    const int barid = 1 + wgi;
+    // column partial buffer of this warpgroup: [chunk][warp q][g][c4 * 8 + k * 2 + j]; the two 16-byte halves of a
+    // thread's 32 bytes are swapped for odd g (conflict-free stores), the readers undo it
+    const uint32_t cp_wg = smem_u32(sCP) + wgi * 16384;
+    const uint32_t cp_st = cp_wg + (q * 8 + g) * 128 + c4 * 32;
+    const uint32_t cp_st0 = cp_st + ((g & 1) << 4), cp_st1 = cp_st + (((g & 1) ^ 1) << 4);
+    const int H = (R - 1) >> 1;  // full tiles per row block
+    const bool ragged = (p.cols & 127) != 0;
+    int gt = 0;
+    for (int u = blockIdx.x; u < nunits; u += gridDim.x) {
+      const UnitInfo ui = decode_unit(p, u);
+      const int rb = ui.g0 >> 7;
+      unsigned long long racc[4] = {0ull, 0ull, 0ull, 0ull};
+      for (int t = ui.t0; t < ui.t1; ++t, ++gt) {
+        if ((gt & 1) != pair) continue;
+        mbar_wait_a(a_s_full, (gt >> 1) & 1);
+        tc_fence_after();
+        const int o = 2 * t + half;
+        const uint32_t taddr = tmem + tlane + pair * BN + half * 128;
+        if (o >= p.band) {  // odd band: the second half of the last stage is not part of it
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive_a(a_s_empty);
+          continue;
+        }
+        const int b = (rb + o) % R;
+        const bool cols = o >= 1 && o <= H;
+        const bool masked = o == 0 || (ragged && (rb == R - 1 || b == R - 1));
+        const int row_w = ui.g0 + q * 32;  // global rows / columns: padding test against p.cols
+        if (!cols) {
+          sym_tile<true, false>(taddr, p, racc, a_s_empty, lane, 0, 0, barid, row_w, b * 128, o == 0);
+          continue;
+        }
+        if (masked)
+          sym_tile<true, true>(taddr, p, racc, a_s_empty, lane, cp_st0, cp_st1, barid, row_w, b * 128, false);
+        else
+          sym_tile<false, true>(taddr, p, racc, a_s_empty, lane, cp_st0, cp_st1, barid, row_w, b * 128, false);
+        named_bar_sync(barid, 128);
+        if (q < 2) {
+          // readers: column pair rd = q * 32 + lane of the tile (chunk rd >> 4, k = (rd >> 2) & 3, c4 = rd & 3), its
+          // 32 partials (4 warps x 8 lane groups) summed in a fixed order
+          const int rd = q * 32 + lane;
+          const int rd_k = (rd >> 2) & 3;
+          const uint32_t cp_rd = cp_wg + (rd >> 4) * 4096 + (rd & 3) * 32;
+          const int rd_col = (rd >> 4) * 32 + 8 * rd_k + 2 * (rd & 3);
+          unsigned long long s2 = pack_f32x2(0.f, 0.f);
+#pragma unroll
+          for (int w = 0; w < 4; ++w)
+#pragma unroll
+            for (int gg = 0; gg < 8; ++gg) {
+              unsigned long long x;
+              asm volatile("ld.shared.b64 %0, [%1];"
+                           : "=l"(x)
+                           : "r"(cp_rd + (w * 8 + gg) * 128 + ((rd_k * 8) ^ ((gg & 1) << 4))));
+              s2 = add_f32x2(s2, x);
+            }
+          float c0, c1;
+          unpack_f32x2(s2, c0, c1);
+          *reinterpret_cast<float2*>(p.colpart + static_cast<size_t>(o - 1) * p.part_stride + b * 128 + rd_col) =
+              make_float2(c0, c1);
+        }
+      }
+      // row sums: the packed halves, then the 4 lanes of a row group (butterfly: identical bits in all four)
+      float rs[4];
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        float x0, x1;
+        unpack_f32x2(racc[r], x0, x1);
+        rs[r] = x0 + x1;
+        rs[r] += __shfl_xor_sync(0xffffffffu, rs[r], 1);
+        rs[r] += __shfl_xor_sync(0xffffffffu, rs[r], 2);
+      }
+#pragma unroll
+      for (int r = 0; r < 4; ++r) {
+        const int row_l = q * 32 + g + 8 * r;
+        if (c4 == r && row_l < ui.nvalid)
+          p.part_l[static_cast<size_t>(ui.ch * 4 + wgi) * p.part_stride + ui.lrow0 + row_l] = rs[r];
+      }
+    }
   }
   tc_fence_before();
   __syncthreads();
