@@ -18,7 +18,7 @@
  *    global mutable state that affects results: entry points are re-entrant (autograd calls bwd from its own thread;
  *    the library only memoises - a per-thread cache of encoded TMA descriptors, per-kernel attribute bits - and
  *    keeps the opt-in profiling counters of ssvb_profile_enable).  A/B switches for measurements and tests are read
- *    from the environment once per process (SSVB_NO_PDL, SSVB_GEMM_NO_TMA_STORE, SSVB_SK_NO_BATCH, SSVB_BARLOW_NO_X2,
+ *    from the environment once per process (SSVB_GEMM_NO_TMA_STORE, SSVB_SK_NO_BATCH, SSVB_BARLOW_NO_X2,
  *    SSVB_BARLOW_NO_FUSED_BWD, SSVB_SWAV_NO_CE4, SSVB_SWAV_NO_FUSED_CODES: each selects the previous form of one
  *    kernel sequence, same results within rounding; unset = the shipped path);
  *  - `loss` and `grad_out` are device scalars (fp32) so no device->host sync is ever needed;

@@ -447,9 +447,6 @@ int ssvb_moco_fwd(const float* query, const float* keys, const float* queue, con
     p.dacc = ws.dacc;
     p.ld_dacc = static_cast<int>(dpad);
     p.use_atomic = p.nchunks > 1;  // (ws.dacc was zeroed by the prep kernel)
-#ifdef SSVB_DBG_TIMING
-    if (const char* e = getenv("SSVB_DBG_PTR")) p.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
-#endif
     SSVB_TRY(launch_sim_bwd(SIM_MOCO, sv.qhat, npad, qb, k, dpad, p, s));
     moco_fused_finalize_kernel<<<static_cast<unsigned>(ceil_div(n, 8)), 256, 0, s>>>(
         ws.part_l, 4 * p.nchunks, p.part_stride, static_cast<int>(n), static_cast<int>(dpad), sv.pos, c, c, ws.dacc,

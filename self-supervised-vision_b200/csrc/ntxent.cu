@@ -238,9 +238,6 @@ int ssvb_ntxent_fwd(const float* zi, const float* zj, int64_t n, int64_t d, int6
   p.part_m = ws.part_m;
   p.part_l = ws.part_l;
   p.part_stride = static_cast<int>(round_up(pl.m, 256));
-#ifdef SSVB_DBG_TIMING
-  if (const char* e = getenv("SSVB_DBG_PTR")) p.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
-#endif
   // FIXED mode needs no running max, so S = S^T is exploited: every tile is computed once and also yields the row
   // sums of its mirror (column partials after the row partials, summed by the finalize in index order)
   int nparts;
@@ -302,9 +299,6 @@ int ssvb_ntxent_bwd(const float* zi, const float* zj, int64_t n, int64_t d, int6
   p.dacc = ws.dacc;
   p.ld_dacc = static_cast<int>(pl.dpad);
   p.use_atomic = p.nchunks > 1;
-#ifdef SSVB_DBG_TIMING
-  if (const char* e = getenv("SSVB_DBG_PTR")) p.dbg = reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0));
-#endif
   if (p.use_atomic) SSVB_CUDA(cudaMemsetAsync(ws.dacc, 0, pl.m * pl.dpad * sizeof(float), s));
   SSVB_TRY(launch_sim_bwd(pl.mode, sv.zhat, pl.mpad, sv.zhat, pl.mpad, pl.dpad, p, s));
   {

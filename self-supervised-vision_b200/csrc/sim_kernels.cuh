@@ -40,7 +40,6 @@ struct SimParams {
   float* dacc;           // [local rows x ld_dacc] fp32
   int ld_dacc;
   int use_atomic;  // nchunks > 1: red.add into a zeroed dacc
-  unsigned long long* dbg;  // SSVB_DBG_TIMING builds only
   int opf16;  // similarity operands staged as fp16 (normalised rows) instead of bf16
   int dhalf;  // backward, dpad = 256 only: which 128-column half of dZ this launch produces
 };
@@ -80,42 +79,12 @@ __device__ __forceinline__ UnitInfo decode_unit(const SimParams& p, int u) {
   return ui;
 }
 
-// phase timing (timing experiments only): block 0, first lane of the first math warp / of the MMA warp accumulate
-// clock64 deltas per phase into p.dbg[0..15]
-#ifdef SSVB_DBG_TIMING
-#define SSVB_T0() long long _t_prev = clock64()
-#define SSVB_TP(slot) do { const long long _t_now = clock64(); _t_acc[slot] += _t_now - _t_prev; _t_prev = _t_now; } while (0)
-#else
-#define SSVB_T0() do {} while (0)
-#define SSVB_TP(slot) do {} while (0)
-#endif
-
-__device__ __forceinline__ float ex2_poly3(float x);
-// ---- timing-experiment knobs (tools/ab_bench.sh): each one REMOVES a piece of work, results become wrong ----
-#ifdef SSVB_DBG_NOEXP
-#define SSVB_EX2(x) (x)
-#else
-#define SSVB_EX2(x) ex2f(x)
-#endif
-#ifndef SSVB_POLY_MOD_FWD
-#define SSVB_POLY_MOD_FWD 3   // masked (rare) tiles only: every 3rd element on the scalar polynomial
-#endif
-// FIXED mode hot loops: of every SSVB_POLY_*_MOD consecutive PAIRS, the first SSVB_POLY_*_CNT take the packed
-// polynomial exp2 and the rest two MUFU.EX2 (CNT = 0: MUFU only).  MUFU issues through the MIO queue at 16 / clk / SM
-// and is co-critical with the tensor pipe in both kernels (ncu: mio_throttle on MUFU.EX2), so a share of the
-// exponentials moves to the FMA pipe; tuned by A/B builds (profiles/r2_tuning_log.md).
-#ifndef SSVB_POLY_FWD_MOD
-#define SSVB_POLY_FWD_MOD 2
-#endif
-#ifndef SSVB_POLY_FWD_CNT
-#define SSVB_POLY_FWD_CNT 1
-#endif
-#ifndef SSVB_POLY_BWD_MOD
-#define SSVB_POLY_BWD_MOD 3
-#endif
-#ifndef SSVB_POLY_BWD_CNT
-#define SSVB_POLY_BWD_CNT 1
-#endif
+// FIXED mode hot loops: of every kPolyFwdPeriod (forward) / kPolyBwdPeriod (backward) consecutive PAIRS of
+// exponentials, the first takes the packed polynomial exp2 and the rest two MUFU.EX2.  MUFU issues through the MIO
+// queue at 16 / clk / SM and is co-critical with the tensor pipe in both kernels (ncu: mio_throttle on MUFU.EX2), so a
+// share of the exponentials moves to the FMA pipe (shares measured in profiles/r2_tuning_log.md).
+constexpr int kPolyFwdPeriod = 2;
+constexpr int kPolyBwdPeriod = 3;
 
 // exp2 of two values on the FMA pipe with packed instructions (Cody-Waite split + degree-3 minimax, max rel. error
 // 7.5e-5): 6 FADD2/FFMA2 + 2 IMAD per pair = 4 issue slots per element and no MUFU slot.  Valid for x > -126.
@@ -146,12 +115,10 @@ __device__ __forceinline__ void lds_v4(uint32_t saddr, unsigned long long& lo, u
 // forward
 // =====================================================================================================
 // Forward tile width.  256: two 256-column S buffers, a warpgroup PAIR shares a tile (one 128-column half each) and the
-// buffer is handed back after 3/4 of the pair's math (default).  128: FOUR 128-column S buffers, each softmax warpgroup
-// owns a whole tile in its own buffer (more independent MMA -> softmax streams); kept as a build option, measured slower.
-#ifndef SSVB_FWD_BN
-#define SSVB_FWD_BN 256   // measured (profiles/r2_tuning_log.md): 128 is 4 % slower (16 instead of 8 MMAs + commits per 256 columns on the one issuing thread)
-#endif
-constexpr int kFwdBN = SSVB_FWD_BN;
+// buffer is handed back after 3/4 of the pair's math.  128: FOUR 128-column S buffers, each softmax warpgroup owns a
+// whole tile in its own buffer (more independent MMA -> softmax streams).  Measured (profiles/r2_tuning_log.md): 128 is
+// 4 % slower (16 instead of 8 MMAs + commits per 256 columns on the one issuing thread).
+constexpr int kFwdBN = 256;
 template <int KB>
 struct FwdCfg {
   // d <= 128 (KB <= 2): BN = kFwdBN.  128 < d <= 256 (KB = 4, dpad = 256): 128-column tiles (four S buffers) and a
@@ -167,31 +134,16 @@ struct FwdCfg {
 
 template <int MODE, bool MASKED>
 __device__ __forceinline__ void fwd_tile(uint32_t taddr, const SimParams& p, int a_glob, int j0, float& m,
-                                         float (&l)[4], uint32_t s_empty_bar, int lane
-#ifdef SSVB_DBG_TIMING
-                                         , long long (&_t_acc)[8], long long& _t_prev
-#endif
-                                         ) {
+                                         float (&l)[4], uint32_t s_empty_bar, int lane) {
   uint32_t v[2][32];
   unsigned long long l2[2] = {pack_f32x2(0.f, 0.f), pack_f32x2(0.f, 0.f)};  // packed row-sum accumulators
-#ifndef SSVB_DBG_NOLD
   tmem_ld_x32(taddr, v[0]);
-#else
-#pragma unroll
-  for (int i = 0; i < 32; ++i) { v[0][i] = __float_as_uint(1e-3f * (i + lane)); v[1][i] = __float_as_uint(2e-3f * (i + lane)); }
-#endif
 #pragma unroll
   for (int cc = 0; cc < 4; ++cc) {
     uint32_t(&cur)[32] = v[cc & 1];
-    SSVB_TP(3);  // exp / sum work of the previous chunk
-#ifndef SSVB_DBG_NOLD
     tmem_ld_wait_regs(cur);
-#endif
-    SSVB_TP(2);  // waiting for the TMEM load
     if (cc < 3) {
-#ifndef SSVB_DBG_NOLD
       tmem_ld_x32(taddr + (cc + 1) * 32, v[(cc + 1) & 1]);
-#endif
     } else {
       // the S buffer is fully in registers: hand it back to the MMA warp
       tc_fence_before();
@@ -204,12 +156,11 @@ __device__ __forceinline__ void fwd_tile(uint32_t taddr, const SimParams& p, int
       // logit: no scale/shift FFMA.  Per pair: two MUFU.EX2 or one packed polynomial, one packed row-sum FADD2.
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
-        const bool poly = (i % SSVB_POLY_FWD_MOD) < SSVB_POLY_FWD_CNT;
         unsigned long long e2;
-        if (poly) {
+        if (i % kPolyFwdPeriod == 0) {
           e2 = ex2_poly3_x2(pack_f32x2(__uint_as_float(cur[2 * i]), __uint_as_float(cur[2 * i + 1])));
         } else {
-          e2 = pack_f32x2(SSVB_EX2(__uint_as_float(cur[2 * i])), SSVB_EX2(__uint_as_float(cur[2 * i + 1])));
+          e2 = pack_f32x2(ex2f(__uint_as_float(cur[2 * i])), ex2f(__uint_as_float(cur[2 * i + 1])));
         }
         l2[i & 1] = add_f32x2(l2[i & 1], e2);
       }
@@ -221,8 +172,7 @@ __device__ __forceinline__ void fwd_tile(uint32_t taddr, const SimParams& p, int
           const int col = colbase + i;
           if (col == a_glob || col >= p.cols) t = -INFINITY;
         }
-        const bool poly = !MASKED && SSVB_POLY_MOD_FWD > 0 && (i % (SSVB_POLY_MOD_FWD > 0 ? SSVB_POLY_MOD_FWD : 1)) == 1;
-        l[i & 3] += poly ? ex2_poly3(t) : SSVB_EX2(t);
+        l[i & 3] += ex2f(t);
       }
     } else {
       float x[32];
@@ -347,14 +297,12 @@ sim_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         tc_fence_after();
         if (elect_one()) {
           const uint32_t bbase = smem_u32(sB + st * C::B_BYTES);
-#ifndef SSVB_DBG_FWD_NOS
 #pragma unroll
           for (int kb = 0; kb < KB; ++kb)
 #pragma unroll
             for (int k4 = 0; k4 < 4; ++k4)
               umma_ss(tmem + buf * BN, desc_kmajor(abase + kb * (128 * 128) + k4 * 32),
                       desc_kmajor(bbase + kb * (BN * 128) + k4 * 32), IDESC, (kb | k4) != 0);
-#endif
           umma_commit(&b_empty[st]);
           umma_commit(&s_full[buf]);
           if (t == ui.t1 - 1) umma_commit(&a_empty[0]);
@@ -374,10 +322,6 @@ sim_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     int gt = 0;
     const int my_buf = NBUF == 2 ? pair : wgi;
     const uint32_t a_s_full = smem_u32(&s_full[my_buf]), a_s_empty = smem_u32(&s_empty[my_buf]);  // hoisted (see bwd)
-#ifdef SSVB_DBG_TIMING
-    long long _t_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#endif
-    SSVB_T0();
     for (int u = blockIdx.x; u < nunits; u += gridDim.x) {
       const UnitInfo ui = decode_unit(p, u);
       const int a_glob = ui.g0 + row_l;
@@ -388,24 +332,15 @@ sim_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         // BN = 128: tile t belongs to warpgroup (t & 3) alone (its own S buffer)
         if (NBUF == 2 ? ((gt & 1) != pair) : ((gt & 3) != wgi)) continue;
         const int buf = NBUF == 2 ? pair : wgi;
-        SSVB_TP(0);  // loop / other
         mbar_wait_a(a_s_full, (gt / NBUF) & 1);
         tc_fence_after();
-        SSVB_TP(1);  // wait s_full
         const int j0 = t * BN + (NBUF == 2 ? half * 128 : 0);
         const bool special = (MODE != SIM_MOCO && j0 < ui.g0 + 128 && j0 + 128 > ui.g0) || (j0 + 128 > p.cols);
         const uint32_t taddr = tmem + tlane + buf * BN + (NBUF == 2 ? half * 128 : 0);
-#ifdef SSVB_DBG_TIMING
-        if (special)
-          fwd_tile<MODE, true>(taddr, p, a_glob, j0, m, l, a_s_empty, lane, _t_acc, _t_prev);
-        else
-          fwd_tile<MODE, false>(taddr, p, a_glob, j0, m, l, a_s_empty, lane, _t_acc, _t_prev);
-#else
         if (special)
           fwd_tile<MODE, true>(taddr, p, a_glob, j0, m, l, a_s_empty, lane);
         else
           fwd_tile<MODE, false>(taddr, p, a_glob, j0, m, l, a_s_empty, lane);
-#endif
       }
       if (row_l < ui.nvalid) {
         const size_t o = static_cast<size_t>(ui.ch * 4 + wgi) * p.part_stride + ui.lrow0 + row_l;
@@ -413,10 +348,6 @@ sim_fwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (MODE != SIM_NTX_FIXED) p.part_m[o] = m;
       }
     }
-#ifdef SSVB_DBG_TIMING
-    if (p.dbg && blockIdx.x == 0 && warp == 4 && lane == 0)
-      for (int i = 0; i < 8; ++i) p.dbg[16 + i] = static_cast<unsigned long long>(_t_acc[i]);
-#endif
   }
   tc_fence_before();
   __syncthreads();
@@ -506,10 +437,10 @@ __device__ __forceinline__ void sym_tile(uint32_t taddr, const SimParams& p, uns
             e[j] = ex2f(off ? -INFINITY : __uint_as_float(cur[idx + j]));
           }
           e2 = pack_f32x2(e[0], e[1]);
-        } else if (((4 * k + r) % SSVB_POLY_FWD_MOD) < SSVB_POLY_FWD_CNT) {
+        } else if ((4 * k + r) % kPolyFwdPeriod == 0) {
           e2 = ex2_poly3_x2(pack_f32x2(__uint_as_float(cur[idx]), __uint_as_float(cur[idx + 1])));
         } else {
-          e2 = pack_f32x2(SSVB_EX2(__uint_as_float(cur[idx])), SSVB_EX2(__uint_as_float(cur[idx + 1])));
+          e2 = pack_f32x2(ex2f(__uint_as_float(cur[idx])), ex2f(__uint_as_float(cur[idx + 1])));
         }
         racc[r] = add_f32x2(racc[r], e2);
         if (COLS) cacc[k] = r == 0 ? e2 : add_f32x2(cacc[k], e2);
@@ -752,26 +683,10 @@ struct BwdCfg {
   static constexpr int T_W = 384;
 };
 
-// exp2 on the FMA/ALU pipes (Cody-Waite split + degree-3 minimax, max rel. error 7.5e-5): takes a share of the
-// exponentials off the 16-op/clk MUFU unit, which is what bounds the forward kernel at d = 128.  Valid for x > -126.
-__device__ __forceinline__ float ex2_poly3(float x) {
-  const float magic = 12582912.f;  // 1.5 * 2^23: x + magic rounds x to the nearest integer in the low mantissa bits
-  const float r = x + magic;
-  const float f = x - (r - magic);  // f in [-0.5, 0.5]
-  float p = fmaf(f, 5.517166745e-2f, 2.426111221e-1f);
-  p = fmaf(p, f, 6.932609858e-1f);
-  p = fmaf(p, f, 9.999280736e-1f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(r) << 23));
-}
-#ifndef SSVB_POLY_MOD_BWD
-#define SSVB_POLY_MOD_BWD 0  // share of backward exponentials on the polynomial path (measured: no gain, off)
-#endif
-
 // weights of 32 consecutive columns [cb, cb+32) of one row: sv = S values, pk = packed bf16 pairs out
 template <int MODE, bool MASKED, bool OPF16>
 __device__ __forceinline__ void bwd_weights32(const uint32_t (&sv)[32], uint32_t (&pk)[16], const SimParams& p,
                                               int a_glob, int colbase, float rs, uint32_t cs32, float& wsum) {
-#ifndef SSVB_BWD_SCALAR_MATH
   if (MODE == SIM_NTX_FIXED && !MASKED) {
     // issue-bound loop.  Operands are pre-scaled (the S accumulator is the log2-domain logit): per pair two MUFU.EX2
     // (or one packed polynomial), FADD2 (row + column factor), FMUL2, one pack -> 2.5 issue slots per element.
@@ -784,12 +699,11 @@ __device__ __forceinline__ void bwd_weights32(const uint32_t (&sv)[32], uint32_t
 #pragma unroll
       for (int e = 0; e < 2; ++e) {
         const int i = i2 * 2 + e;  // pair index: columns 2i, 2i+1
-        const bool poly = (i % SSVB_POLY_BWD_MOD) < SSVB_POLY_BWD_CNT;
         unsigned long long e2;
-        if (poly) {
+        if (i % kPolyBwdPeriod == 0) {
           e2 = ex2_poly3_x2(pack_f32x2(__uint_as_float(sv[2 * i]), __uint_as_float(sv[2 * i + 1])));
         } else {
-          e2 = pack_f32x2(SSVB_EX2(__uint_as_float(sv[2 * i])), SSVB_EX2(__uint_as_float(sv[2 * i + 1])));
+          e2 = pack_f32x2(ex2f(__uint_as_float(sv[2 * i])), ex2f(__uint_as_float(sv[2 * i + 1])));
         }
         const unsigned long long w2 = mul_f32x2(e2, add_f32x2(rs2, cu[e]));
         float w0, w1;
@@ -799,7 +713,6 @@ __device__ __forceinline__ void bwd_weights32(const uint32_t (&sv)[32], uint32_t
     }
     return;
   }
-#endif
 #pragma unroll
   for (int i4 = 0; i4 < 8; ++i4) {
     float csv[4] = {0.f, 0.f, 0.f, 0.f};
@@ -817,8 +730,7 @@ __device__ __forceinline__ void bwd_weights32(const uint32_t (&sv)[32], uint32_t
       float wv;
       if (MODE == SIM_NTX_FIXED) {
         const float x = fmaf(s, p.c, -p.shift);
-        const bool poly = !MASKED && SSVB_POLY_MOD_BWD > 0 && (i % (SSVB_POLY_MOD_BWD > 0 ? SSVB_POLY_MOD_BWD : 1)) == 1;
-        wv = (poly ? ex2_poly3(x) : SSVB_EX2(x)) * (rs + csv[e]);
+        wv = ex2f(x) * (rs + csv[e]);
       } else if (MODE == SIM_NTX_ONLINE) {
         const float t = s * p.c;
         wv = ex2f(t - rs) + ex2f(t - csv[e]);
@@ -936,14 +848,12 @@ sim_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           tc_fence_after();
           if (elect_one()) {
             const uint32_t bbase = smem_u32(sB + st * C::B_BYTES);
-#ifndef SSVB_DBG_NOS
 #pragma unroll
             for (int kb = 0; kb < KB; ++kb)
 #pragma unroll
               for (int k4 = 0; k4 < 4; ++k4)
                 umma_ss(tmem + C::T_S + buf * BN, desc_kmajor(abase + kb * (128 * 128) + k4 * 32),
                         desc_kmajor(bbase + kb * (BN * 128) + k4 * 32), IDESC_S, (kb | k4) != 0);
-#endif
             umma_commit(&s_full[buf]);
             if (t == ui.t1 - 1) umma_commit(a_empty);  // last reader of this unit's A tile
           }
@@ -963,13 +873,11 @@ sim_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           tc_fence_after();
           if (elect_one()) {
             const uint32_t bbase = smem_u32(sB + st * C::B_BYTES);
-#ifndef SSVB_DBG_NOD
 #pragma unroll
             for (int k = 0; k < BN / 16; ++k)
               umma_ts(tmem + C::T_DZ, tmem + C::T_W + buf * 64 + k * 8,
                       desc_mnmajor(bbase + (KB > 2 ? p.dhalf * 2 * (BN * 128) : 0) + k * (16 * 128), BN * 128), IDESC_D,
                       (t > ui.t0 || k > 0) ? 1u : 0u);
-#endif
             umma_commit(&b_empty[st]);
             umma_commit(&w_empty[buf]);
             if (t == ui.t1 - 1) umma_commit(dz_full);
@@ -993,10 +901,6 @@ sim_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const uint32_t a_w_full = smem_u32(&w_full[pair]), a_w_empty = smem_u32(&w_empty[pair]);
     const uint32_t a_dz_full = smem_u32(dz_full), a_dz_empty = smem_u32(dz_empty);
     const uint32_t a_sC = smem_u32(sC) + half * 64 * 4;
-#ifdef SSVB_DBG_TIMING
-    long long _t_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#endif
-    SSVB_T0();
     for (int u = blockIdx.x; u < nunits; u += gridDim.x, ++ucount) {
       const UnitInfo ui = decode_unit(p, u);
       const int a_glob = ui.g0 + row_l;
@@ -1007,29 +911,20 @@ sim_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       for (int t = ui.t0; t < ui.t1; ++t, ++gt) {
         if ((gt & 1) != pair) continue;
         const int st = gt % NSTAGE;
-        SSVB_TP(0);  // loop overhead / other
         // no separate wait on b_full: S(t) was issued only after the MMA warp observed b_full[st], so observing
         // s_full(t) also orders this warp after the TMA / bulk-copy writes of the B tile and its column statistics
-        SSVB_TP(1);
         mbar_wait_a(a_s_full, (gt >> 1) & 1);
         tc_fence_after();
-        SSVB_TP(2);  // wait s_full
         const uint32_t t_s = tmem + tlane + C::T_S + pair * BN + half * 64;
         uint32_t sv[2][32];
-#ifndef SSVB_DBG_NOLD
         tmem_ld_x32(t_s, sv[0]);
         tmem_ld_x32(t_s + 32, sv[1]);
         tmem_ld_wait_regs(sv[0]);
         tmem_ld_wait_regs(sv[1]);
-#else
-#pragma unroll
-        for (int i = 0; i < 32; ++i) { sv[0][i] = __float_as_uint(1e-3f * (i + lane)); sv[1][i] = sv[0][i]; }
-#endif
         // this half of the S tile is in registers: give the buffer back so S(t+2) can be issued right away
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_a(a_s_empty);
-        SSVB_TP(3);  // tmem loads + release
         const int j0 = t * BN + half * 64;
         const bool special = (MODE != SIM_MOCO) ? ((j0 < ui.g0 + 128) && (j0 + 64 > ui.g0)) : (j0 + 64 > p.cols);
         const uint32_t t_w = tmem + tlane + C::T_W + pair * 64 + half * 32;
@@ -1045,18 +940,14 @@ sim_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           bwd_weights32<MODE, false, OPF16>(sv[0], pk[0], p, a_glob, j0, rs, cs, lsum);
           bwd_weights32<MODE, false, OPF16>(sv[1], pk[1], p, a_glob, j0 + 32, rs, cs + CSTEP, lsum);
         }
-        SSVB_TP(4);  // 64 weights
         mbar_wait_a(a_w_empty, ((gt >> 1) & 1) ^ 1);
         tc_fence_after();
-        SSVB_TP(5);  // wait w_empty
         tmem_st_x16(t_w, pk[0]);
         tmem_st_x16(t_w + 16, pk[1]);
-        SSVB_TP(6);  // stores issued
         tmem_st_wait();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_a(a_w_full);
-        SSVB_TP(7);  // st drain + arrive
       }
       if (MODE == SIM_MOCO && p.part_l != nullptr && valid)
         p.part_l[static_cast<size_t>(ui.ch * 4 + wgi) * p.part_stride + ui.lrow0 + row_l] = lsum;
@@ -1088,10 +979,6 @@ sim_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       __syncwarp();
       if (lane == 0) mbar_arrive_a(a_dz_empty);
     }
-#ifdef SSVB_DBG_TIMING
-    if (p.dbg && blockIdx.x == 0 && warp == 4 && lane == 0)
-      for (int i = 0; i < 8; ++i) p.dbg[i] = static_cast<unsigned long long>(_t_acc[i]);
-#endif
   }
   tc_fence_before();
   __syncthreads();

@@ -251,127 +251,11 @@ __global__ void sk_pass_kernel(const float* __restrict__ s, int64_t b, int k, in
   }
 }
 
-// Fast path (K <= 3072, K % 4 == 0, 16-byte aligned rows): one warp per row, the whole row lives in registers
-// (24 float4 per lane, all loads issued up front -> 12 KB in flight per warp), column sums accumulate in registers
-// across the rows of a warp and are combined across the 8 warps of the block in a fixed order through shared memory.
+// float4 per lane of one score row held in registers by the fast path: K <= 32 * 4 * kSkNV = 3072
 constexpr int kSkNV = 24;
-template <int PHASE>
-__global__ void __launch_bounds__(256, 1)
-sk_rowreg_kernel(const float* __restrict__ s, int64_t b, int k, int64_t ld, float inv_eps_log2e,
-                 const float* __restrict__ smax, const float* __restrict__ alpha, float* __restrict__ upart, int kpad,
-                 float* __restrict__ codes, int64_t ldc, float* __restrict__ mpart, float inv_b) {
-  extern __shared__ float sk_smem[];  // [kpad] alpha, then (PHASE != 2) [8][kpad] per-warp column sums
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = blockDim.x >> 5;
-  const int k4 = k >> 2;
-  float* alpha_s = sk_smem;
-  if (PHASE != 0) {
-    for (int c = threadIdx.x; c < k; c += blockDim.x) alpha_s[c] = alpha[c];
-    __syncthreads();
-  }
-  // PHASE 0 needs no prior max pass: every warp keeps a running max Mw of the scores it has seen and rescales its
-  // column sums when Mw grows (online, like a streaming softmax); blocks are combined with exp((M_blk - M)/eps) in
-  // sk_alpha0_kernel, which also publishes the global max for the later passes.
-  float shift = (PHASE == 0) ? 0.f : smax[0] * inv_eps_log2e;
-  float Mw = -INFINITY;
-  float4 acc[kSkNV];
-#pragma unroll
-  for (int j = 0; j < kSkNV; ++j) acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int64_t r = static_cast<int64_t>(blockIdx.x) * nwarp + w; r < b; r += static_cast<int64_t>(gridDim.x) * nwarp) {
-    const float4* row = reinterpret_cast<const float4*>(s + r * ld);
-    float4 e[kSkNV];
-#pragma unroll
-    for (int j = 0; j < kSkNV; ++j) {
-      const int c4 = lane + 32 * j;
-      e[j] = (c4 < k4) ? __ldg(row + c4) : make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
-    }
-    if (PHASE == 0) {
-      float rm = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < kSkNV; ++j) rm = fmaxf(rm, fmaxf(fmaxf(e[j].x, e[j].y), fmaxf(e[j].z, e[j].w)));
-      rm = warp_max(rm);
-      if (rm > Mw) {  // warp-uniform
-        const float sc = ex2f((Mw - rm) * inv_eps_log2e);  // 0 on the first row (Mw = -inf)
-#pragma unroll
-        for (int j = 0; j < kSkNV; ++j) { acc[j].x *= sc; acc[j].y *= sc; acc[j].z *= sc; acc[j].w *= sc; }
-        Mw = rm;
-      }
-      shift = Mw * inv_eps_log2e;
-    }
-    float v = 0.f;
-#pragma unroll
-    for (int j = 0; j < kSkNV; ++j) {
-      e[j].x = ex2f(fmaf(e[j].x, inv_eps_log2e, -shift));
-      e[j].y = ex2f(fmaf(e[j].y, inv_eps_log2e, -shift));
-      e[j].z = ex2f(fmaf(e[j].z, inv_eps_log2e, -shift));
-      e[j].w = ex2f(fmaf(e[j].w, inv_eps_log2e, -shift));
-      if (PHASE != 0) {
-        const int c4 = lane + 32 * j;
-        if (c4 < k4) {
-          const float4 a = reinterpret_cast<const float4*>(alpha_s)[c4];
-          v += (e[j].x * a.x + e[j].y * a.y) + (e[j].z * a.z + e[j].w * a.w);
-        }
-      }
-    }
-    if (PHASE == 0) {
-#pragma unroll
-      for (int j = 0; j < kSkNV; ++j) { acc[j].x += e[j].x; acc[j].y += e[j].y; acc[j].z += e[j].z; acc[j].w += e[j].w; }
-    } else {
-      v = warp_sum(v);
-      if (PHASE == 1) {
-        const float beta = inv_b / v;
-#pragma unroll
-        for (int j = 0; j < kSkNV; ++j) {
-          acc[j].x = fmaf(e[j].x, beta, acc[j].x); acc[j].y = fmaf(e[j].y, beta, acc[j].y);
-          acc[j].z = fmaf(e[j].z, beta, acc[j].z); acc[j].w = fmaf(e[j].w, beta, acc[j].w);
-        }
-      } else {
-        const float iv = 1.f / v;
-        float4* out = reinterpret_cast<float4*>(codes + r * ldc);
-#pragma unroll
-        for (int j = 0; j < kSkNV; ++j) {
-          const int c4 = lane + 32 * j;
-          if (c4 < k4) {
-            const float4 a = reinterpret_cast<const float4*>(alpha_s)[c4];
-            out[c4] = make_float4(e[j].x * a.x * iv, e[j].y * a.y * iv, e[j].z * a.z * iv, e[j].w * a.w * iv);
-          }
-        }
-      }
-    }
-  }
-  if (PHASE != 2) {
-    __shared__ float mw_s[8];
-    float* mine = sk_smem + kpad + w * kpad;
-#pragma unroll
-    for (int j = 0; j < kSkNV; ++j) {
-      const int c4 = lane + 32 * j;
-      if (c4 < k4) reinterpret_cast<float4*>(mine)[c4] = acc[j];
-    }
-    if (PHASE == 0 && lane == 0) mw_s[w] = Mw;
-    __syncthreads();
-    float wsc[8] = {1.f, 1.f, 1.f, 1.f, 1.f, 1.f, 1.f, 1.f};
-    if (PHASE == 0) {
-      float mb = -INFINITY;
-      for (int ww = 0; ww < nwarp; ++ww) mb = fmaxf(mb, mw_s[ww]);
-      for (int ww = 0; ww < nwarp; ++ww) wsc[ww] = (mw_s[ww] == -INFINITY) ? 0.f : ex2f((mw_s[ww] - mb) * inv_eps_log2e);
-      if (threadIdx.x == 0) mpart[blockIdx.x] = mb;
-    }
-    for (int c = threadIdx.x; c < k; c += blockDim.x) {
-      float t = 0.f;
-      for (int ww = 0; ww < nwarp; ++ww) t = fmaf(sk_smem[kpad + ww * kpad + c], wsc[ww], t);
-      upart[static_cast<size_t>(blockIdx.x) * kpad + c] = t;
-    }
-  }
-}
-
-// Fast path v2 (K <= 3072, K % 4 == 0, 16-byte aligned rows): the row stream is decoupled from the math by a TMA ring.
-// One producer warp issues 1-D bulk copies (cp.async.bulk, one whole score row = K*4 bytes per copy, completion on an
-// mbarrier) into a ring of `nst` row slots (up to 16 rows = 192 KB in flight per SM); 8 consumer warps take rows round
-// robin, pull the row from shared memory into registers (24 float4 per lane), hand the slot straight back to the
-// producer, and run the same per-row math as sk_rowreg_kernel (online max in PHASE 0, column sums in registers).
-// The ring is reused for the fixed-order cross-warp combine at the end.
 constexpr int kSkConsumers = 7;  // + 1 producer warp = 8 warps: 2 per SM sub-partition, so 255 registers stay available
 
-// Fast path v2 (K <= 3072, K % 4 == 0, 16-byte aligned rows): the row stream is decoupled from the math by a TMA ring.
+// Fast path (K <= 3072, K % 4 == 0, 16-byte aligned rows): the row stream is decoupled from the math by a TMA ring.
 // One producer warp issues 1-D bulk copies (cp.async.bulk, one whole score row = K*4 bytes per copy, completion on an
 // mbarrier) into a ring of `nst` row slots (up to 16 rows = 192 KB in flight per SM); the scaling vector alpha arrives
 // by one more bulk copy (a serial LDG -> STS prologue cost 27 % of the kernel).  7 consumer warps take rows round
@@ -419,6 +303,9 @@ sk_tma_kernel(const float* __restrict__ s, int64_t b, int k, int64_t ld, float i
   float4 acc[kSkNV];
 #pragma unroll
   for (int j = 0; j < kSkNV; ++j) acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+  // PHASE 0 needs no prior max pass: every warp keeps a running max Mw of the scores it has seen and rescales its
+  // column sums when Mw grows (online, like a streaming softmax); blocks are combined with exp((M_blk - M)/eps) in
+  // sk_alpha0_kernel, which also publishes the global max for the later passes.
   float Mw = -INFINITY;
 
   if (w == kSkConsumers) {
@@ -570,20 +457,12 @@ inline SkRing sk_ring(int kpad) {
   return g;
 }
 template <int PHASE>
-int sk_launch_fast(int grid, size_t smem_unused, cudaStream_t s, const float* scores, int64_t b, int k, int64_t ld, float iel,
-                   const SkWs& ws, float* codes, int64_t ldc, float inv_b, bool pdl = false, int nprob = 1,
-                   int64_t pstride_s = 0, int64_t pstride_c = 0) {
-  (void)smem_unused;
-#ifdef SSVB_SK_ROWREG  // previous fast path (global loads straight into registers), kept for A/B timing
-  const size_t smem = static_cast<size_t>(9) * ws.kpad * 4;
-  SSVB_CUDA(cudaFuncSetAttribute(sk_rowreg_kernel<PHASE>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  sk_rowreg_kernel<PHASE><<<grid, 256, smem, s>>>(scores, b, k, ld, iel, ws.smax, ws.alpha, ws.upart, ws.kpad, codes, ldc,
-                                                  ws.smax_part, inv_b);
-#else
+int sk_launch_fast(int grid, cudaStream_t s, const float* scores, int64_t b, int k, int64_t ld, float iel, const SkWs& ws,
+                   float* codes, int64_t ldc, float inv_b, bool pdl = false, int nprob = 1, int64_t pstride_s = 0,
+                   int64_t pstride_c = 0) {
   const SkRing g = sk_ring(ws.kpad);
   SSVB_CUDA(cudaFuncSetAttribute(sk_tma_kernel<PHASE>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(g.smem)));
-  static const bool no_pdl = getenv("SSVB_NO_PDL") != nullptr;  // A/B switch
-  if (pdl && PHASE != 0 && !no_pdl) {
+  if (pdl && PHASE != 0) {
     // programmatic dependent launch behind the alpha kernel: prologue + first ring-full of rows overlap it
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(static_cast<unsigned>(grid), static_cast<unsigned>(nprob));
@@ -604,7 +483,6 @@ int sk_launch_fast(int grid, size_t smem_unused, cudaStream_t s, const float* sc
         scores, b, k, ld, iel, ws.smax, ws.alpha, ws.upart, ws.kpad, codes, ldc, ws.smax_part, inv_b, g.nst, g.rowf, pstride_s,
         pstride_c);
   }
-#endif
   SSVB_LAUNCH_CHECK();
   return SSVB_OK;
 }
@@ -675,10 +553,7 @@ static int sinkhorn_run_impl(const float* scores, int64_t b, int64_t k, int64_t 
   const bool fast = (k % 4 == 0) && (k <= 128 * kSkNV) && (ld_scores % 4 == 0) && (ld_codes % 4 == 0) &&
                     !(reinterpret_cast<uintptr_t>(scores) & 15) && !(reinterpret_cast<uintptr_t>(codes) & 15);
   static const bool no_batch = getenv("SSVB_SK_NO_BATCH") != nullptr;  // A/B switch
-  bool batch = fast && n_iters > 0 && nprob == kSkMaxProb && (pstride_s % 4 == 0) && (pstride_c % 4 == 0) && !no_batch;
-#ifdef SSVB_SK_ROWREG
-  batch = false;
-#endif
+  const bool batch = fast && n_iters > 0 && nprob == kSkMaxProb && (pstride_s % 4 == 0) && (pstride_c % 4 == 0) && !no_batch;
   if (batched) *batched = batch;
   if (scaling_only && !batch) return SSVB_OK;  // nothing launched: the caller falls back to sinkhorn_run
   if (nprob > 1 && !batch) {
@@ -688,7 +563,6 @@ static int sinkhorn_run_impl(const float* scores, int64_t b, int64_t k, int64_t 
     return SSVB_OK;
   }
   const int np = batch ? nprob : 1;
-  const size_t smem_fast = static_cast<size_t>(9) * ws.kpad * 4;
   // one 8-warp CTA per SM; partial rows [np x fgrid x kpad] (batched: the SMs are split between the problems)
   const int fgrid = batch ? (num_sms() / np > 0 ? num_sms() / np : 1) : num_sms();
   if (!(fast && n_iters > 0)) {  // the fast path finds the max online inside its first pass
@@ -704,7 +578,7 @@ static int sinkhorn_run_impl(const float* scores, int64_t b, int64_t k, int64_t 
     SSVB_LAUNCH_CHECK();
   } else {
     if (fast) {
-      SSVB_TRY(sk_launch_fast<0>(fgrid, smem_fast, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b, false, np,
+      SSVB_TRY(sk_launch_fast<0>(fgrid, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b, false, np,
                                  pstride_s, pstride_c));
       sk_alpha0_kernel<<<alpha_grid, alpha_block, 0, s>>>(ws.upart, ws.smax_part, fgrid, ws.kpad, kk, iel, ws.alpha, ws.smax);
     } else {
@@ -714,7 +588,7 @@ static int sinkhorn_run_impl(const float* scores, int64_t b, int64_t k, int64_t 
     SSVB_LAUNCH_CHECK();
     for (int it = 1; it < n_iters; ++it) {
       if (fast)
-        SSVB_TRY(sk_launch_fast<1>(fgrid, smem_fast, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b, true, np,
+        SSVB_TRY(sk_launch_fast<1>(fgrid, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b, true, np,
                                    pstride_s, pstride_c));
       else SSVB_TRY(sk_launch<1>(regacc, ws.grid, threads, smem, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
       sk_alpha_kernel<<<alpha_grid, alpha_block, 0, s>>>(ws.upart, fast ? fgrid : ws.grid, ws.kpad, kk, ws.alpha);
@@ -724,7 +598,7 @@ static int sinkhorn_run_impl(const float* scores, int64_t b, int64_t k, int64_t 
   if (scaling_only) return SSVB_OK;
   // (n_iters == 0: the final pass follows a fill kernel without the launch_dependents trigger - plain launch)
   if (fast)
-    SSVB_TRY(sk_launch_fast<2>(fgrid, smem_fast, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b, n_iters > 0, np,
+    SSVB_TRY(sk_launch_fast<2>(fgrid, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b, n_iters > 0, np,
                                pstride_s, pstride_c));
   else SSVB_TRY(sk_launch<2>(regacc, ws.grid, threads, smem, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
   return SSVB_OK;
@@ -748,7 +622,6 @@ int sinkhorn_dist_pass(int phase, const float* scores, int64_t b, int64_t b_glob
   // (`fast` must come out the same in all three phases: the caller passes the codes buffer every time)
   const bool fast = (k % 4 == 0) && (k <= 128 * kSkNV) && (ld_scores % 4 == 0) && !(reinterpret_cast<uintptr_t>(scores) & 15) &&
                     (ld_codes % 4 == 0) && !(reinterpret_cast<uintptr_t>(codes) & 15);
-  const size_t smem_fast = static_cast<size_t>(9) * ws.kpad * 4;
   const int fgrid = num_sms();
   const dim3 ablock(32, kSkSlices);
   const unsigned agrid = static_cast<unsigned>(ceil_div(k, 32));
@@ -758,7 +631,7 @@ int sinkhorn_dist_pass(int phase, const float* scores, int64_t b, int64_t b_glob
   }
   if (phase == 0) {
     if (fast) {
-      SSVB_TRY(sk_launch_fast<0>(fgrid, smem_fast, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
+      SSVB_TRY(sk_launch_fast<0>(fgrid, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
       sk_alpha0_kernel<<<agrid, ablock, 0, s>>>(ws.upart, ws.smax_part, fgrid, ws.kpad, kk, iel, u_local, u_local + k, 1);
     } else {
       SSVB_CUDA(cudaMemsetAsync(ws.counter, 0, 16, s));
@@ -771,14 +644,14 @@ int sinkhorn_dist_pass(int phase, const float* scores, int64_t b, int64_t b_glob
     }
     SSVB_LAUNCH_CHECK();
   } else if (phase == 1) {
-    if (fast) SSVB_TRY(sk_launch_fast<1>(fgrid, smem_fast, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
+    if (fast) SSVB_TRY(sk_launch_fast<1>(fgrid, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
     else SSVB_TRY(sk_launch<1>(regacc, ws.grid, threads, smem, s, scores, b, kk, ld_scores, iel, ws, nullptr, 0, inv_b));
     sk_alpha_kernel<<<agrid, ablock, 0, s>>>(ws.upart, fast ? fgrid : ws.grid, ws.kpad, kk, u_local, 1);
     SSVB_LAUNCH_CHECK();
     fill_kernel<<<1, 32, 0, s>>>(u_local + k, 1, 0.f);
     SSVB_LAUNCH_CHECK();
   } else {
-    if (fast) SSVB_TRY(sk_launch_fast<2>(fgrid, smem_fast, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
+    if (fast) SSVB_TRY(sk_launch_fast<2>(fgrid, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
     else SSVB_TRY(sk_launch<2>(regacc, ws.grid, threads, smem, s, scores, b, kk, ld_scores, iel, ws, codes, ld_codes, inv_b));
   }
   return SSVB_OK;
