@@ -6,10 +6,14 @@
 //   dC_aa = 2 (C_aa - 1), dC_ab = 2 lambda C_ab;  dXi~ = Xj~ dC^T / N;  dXj~ = Xi~ dC / N
 //   dx = (dx~ - mean_0(dx~) - x~ * sum_0(dx~ . x~) / (N-1)) / std        [+ row-normalise backward if normalize]
 //
-// Kernels: column statistics (shifted single pass) -> standardise to bf16 -> tcgen05 GEMM with both operands
-// consumed MN-major in place (no transposed copies) and a fused epilogue that reduces the loss and emits dC in
-// bf16 (the D x D fp32 matrix never reaches HBM) -> two tcgen05 GEMMs for the backward -> column reductions +
-// standardise-backward.
+// Forward, both views per launch: column statistics (shifted single pass) -> standardise to bf16 -> tcgen05 GEMM with
+// both operands consumed MN-major in place (no transposed copies) and a fused epilogue that reduces the loss, emits dC in
+// bf16 (the D x D fp32 matrix never reaches HBM) and takes the row / column sums of dC .* C -> one kernel that finishes
+// the loss and q_i / q_j.
+// Backward: ONE dual tcgen05 GEMM (dTi = Xj~ dC^T / n, dTj = Xi~ dC / n) whose epilogue applies the closed-form
+// standardise-backward and writes dzi / dzj.  normalize = 1 (and the row-store epilogue) goes through fp32 dT instead:
+// the dual GEMM writes dT (its epilogue also takes the column partials when they fit, else a separate reduction pass
+// does) -> column finalize -> finish kernel with the row-normalise backward, both views per launch.
 #include "gemm_host.cuh"
 
 using namespace ssvb;
@@ -226,11 +230,6 @@ __device__ __forceinline__ void col_stats4_body(const float* __restrict__ x, int
   }
 }
 
-__global__ void __launch_bounds__(256)
-col_stats4_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict__ inv_row, int64_t n, int d,
-                  float* __restrict__ part) {
-  col_stats4_body(x, ldx, inv_row, n, d, part);
-}
 // Both views of the Barlow forward in ONE launch (view = blockIdx.z / blockIdx.y of the kernels below): the launch ramp,
 // tail and dependency gap of three kernels are paid once instead of twice (profiles/r2_tuning_log.md §6).
 struct TwoViews {
@@ -246,30 +245,6 @@ col_stats4_x2_kernel(TwoViews v, int64_t n, int d, float* __restrict__ part, int
   const bool second = blockIdx.z != 0;
   col_stats4_body(second ? v.x1 : v.x0, second ? v.ld1 : v.ld0, second ? v.inv1 : v.inv0, n, d,
                   part + (second ? view_stride : 0));
-}
-
-// MODE 0: mean, 1/std (unbiased)   MODE 1: mean_0(dT), sum_0(dT x~)/(n-1)
-template <int MODE>
-__global__ void col_finalize_kernel(const float* __restrict__ part, int nsplit, const float* __restrict__ x,
-                                    const float* __restrict__ inv_row, int64_t n, int d, float* __restrict__ out0,
-                                    float* __restrict__ out1) {
-  const int col = blockIdx.x * blockDim.x + threadIdx.x;
-  if (col >= d) return;
-  float s1 = 0.f, s2 = 0.f;
-  for (int i = 0; i < nsplit; ++i) {
-    s1 += part[(static_cast<int64_t>(i) * 2 + 0) * d + col];
-    s2 += part[(static_cast<int64_t>(i) * 2 + 1) * d + col];
-  }
-  const float fn = static_cast<float>(n);
-  if (MODE == 0) {
-    const float v0 = x[col] * (inv_row ? inv_row[0] : 1.f);
-    const float var = (s2 - s1 * s1 / fn) / (fn - 1.f);
-    out0[col] = v0 + s1 / fn;
-    out1[col] = rsqrtf(var);
-  } else {
-    out0[col] = s1 / fn;
-    out1[col] = s2 / (fn - 1.f);
-  }
 }
 
 // forward statistics of both views: blockIdx.y = view
@@ -308,7 +283,7 @@ __global__ void col_finalize_x2_kernel(const float* __restrict__ part, int64_t v
 // MODE 1 finalize for MANY stripes (the GEMM epilogue's partials: one stripe per 32 rows): block (32 columns x 8 stripe
 // phases), fixed-order combine.  out0 = mean_0(dT), out1 = sum_0(dT x~) / (n - 1).
 __global__ void col_finalize_wide_kernel(const float* __restrict__ part, int nsplit, int64_t n, int d,
-                                         float* __restrict__ out0, float* __restrict__ out1, int64_t part_view_stride = 0) {
+                                         float* __restrict__ out0, float* __restrict__ out1, int64_t part_view_stride) {
   // blockIdx.y = view (two-view launch): partials `part_view_stride` apart, outputs [out0 | out1] pairs 2 * d apart
   part += blockIdx.y * part_view_stride;
   out0 += blockIdx.y * 2 * static_cast<int64_t>(d);
@@ -636,29 +611,6 @@ int check_shape(int64_t n, int64_t d) {
   return SSVB_OK;
 }
 
-int stats_and_standardize(const float* x, int64_t ld, int normalize, int64_t n, int64_t d, float* inv_row, float* mean,
-                          float* rstd, __nv_bfloat16* xt, float* colpart, cudaStream_t s) {
-  const float* inv = nullptr;
-  if (normalize) {
-    row_invnorm_kernel<<<static_cast<unsigned>(ceil_div(n, 8)), 256, 0, s>>>(x, n, static_cast<int>(d), ld, inv_row);
-    SSVB_LAUNCH_CHECK();
-    inv = inv_row;
-  }
-  dim3 grid(static_cast<unsigned>(ceil_div(d, 128)), kStatSplit), block(32, 8);
-  col_stats4_kernel<<<grid, block, 0, s>>>(x, ld, inv, n, static_cast<int>(d), colpart);
-  SSVB_LAUNCH_CHECK();
-  col_finalize_kernel<0><<<static_cast<unsigned>(ceil_div(d, 256)), 256, 0, s>>>(colpart, kStatSplit, x, inv, n,
-                                                                                 static_cast<int>(d), mean, rstd);
-  SSVB_LAUNCH_CHECK();
-  const int64_t total = n * (d / 4);
-  int64_t g = ceil_div(total, 256 * 4);
-  const int64_t cap = static_cast<int64_t>(num_sms()) * 16;
-  if (g > cap) g = cap;
-  standardize_kernel<<<static_cast<unsigned>(g), 256, 0, s>>>(x, ld, inv, mean, rstd, n, static_cast<int>(d / 4), xt, d);
-  SSVB_LAUNCH_CHECK();
-  return SSVB_OK;
-}
-
 // Closed-form backward of the batch standardisation.  With x~ = (x - mean) / std (unbiased) and dT = dL/dx~:
 //   dx = (dT - mean_n(dT) - x~ * sum_n(dT x~) / (n - 1)) / std.
 // Here dTi[n, a] = sum_b x~j[n, b] dC[a, b] / n, so mean_n(dTi[., a]) = sum_b dC[a, b] mean_n(x~j[., b]) = 0 (standardised
@@ -710,9 +662,9 @@ __global__ void barlow_fwd_finish_kernel(const float* __restrict__ xrow, int nro
 
 // forward pre-pass of BOTH views in three launches (statistics, finalize, standardize); `xi` heads the two standardised
 // operands (`x_view_stride` elements apart)
-int stats_and_standardize_x2(const float* zi, int64_t ld_zi, const float* zj, int64_t ld_zj, int normalize, int64_t n,
-                             int64_t d, float* inv_i, float* inv_j, TwoStats st, __nv_bfloat16* xi, int64_t x_view_stride,
-                             float* colpart, int64_t part_view_stride, cudaStream_t s) {
+int standardize_both_views(const float* zi, int64_t ld_zi, const float* zj, int64_t ld_zj, int normalize, int64_t n,
+                           int64_t d, float* inv_i, float* inv_j, TwoStats st, __nv_bfloat16* xi, int64_t x_view_stride,
+                           float* colpart, int64_t part_view_stride, cudaStream_t s) {
   TwoViews v{zi, zj, ld_zi, ld_zj, nullptr, nullptr};
   if (normalize) {
     row_invnorm_kernel<<<static_cast<unsigned>(ceil_div(n, 8)), 256, 0, s>>>(zi, n, static_cast<int>(d), ld_zi, inv_i);
@@ -731,7 +683,7 @@ int stats_and_standardize_x2(const float* zi, int64_t ld_zi, const float* zj, in
   SSVB_LAUNCH_CHECK();
   const int64_t total = n * (d / 4);
   int64_t g = ceil_div(total, 256 * 4);
-  const int64_t cap = static_cast<int64_t>(num_sms()) * 8;  // x 2 views = 16 resident-CTA waves' worth, as in the one-view form
+  const int64_t cap = static_cast<int64_t>(num_sms()) * 8;  // x 2 views = 16 resident-CTA waves' worth
   if (g > cap) g = cap;
   standardize_x2_kernel<<<dim3(static_cast<unsigned>(g), 2), 256, 0, s>>>(v, st, n, static_cast<int>(d / 4), xi, x_view_stride,
                                                                         d);
@@ -764,16 +716,9 @@ int ssvb_barlow_fwd(const float* zi, const float* zj, int64_t n, int64_t d, int6
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   BarlowSaved sv = barlow_saved(saved, n, d);
   BarlowWs ws = barlow_ws(workspace, n, d);
-  static const bool no_x2 = getenv("SSVB_BARLOW_NO_X2") != nullptr;  // A/B switch: one view per launch
-  if (no_x2) {
-    SSVB_TRY(stats_and_standardize(zi, ld_zi, normalize, n, d, sv.inv_i, sv.mean_i, sv.rstd_i, sv.xi, ws.colpart, s));
-    SSVB_TRY(stats_and_standardize(zj, ld_zj, normalize, n, d, sv.inv_j, sv.mean_j, sv.rstd_j, sv.xj,
-                                   ws.colpart + ws.view_stride, s));
-  } else {
-    SSVB_TRY(stats_and_standardize_x2(zi, ld_zi, zj, ld_zj, normalize, n, d, sv.inv_i, sv.inv_j,
-                                      TwoStats{sv.mean_i, sv.rstd_i, sv.mean_j, sv.rstd_j}, sv.xi, sv.xj - sv.xi, ws.colpart,
-                                      ws.view_stride, s));
-  }
+  SSVB_TRY(standardize_both_views(zi, ld_zi, zj, ld_zj, normalize, n, d, sv.inv_i, sv.inv_j,
+                                  TwoStats{sv.mean_i, sv.rstd_i, sv.mean_j, sv.rstd_j}, sv.xi, sv.xj - sv.xi, ws.colpart,
+                                  ws.view_stride, s));
   // C = Xi~^T Xj~ / n : contraction over the batch axis, both operands MN-major in place
   GemmParams p{};
   p.M = static_cast<int>(d);
@@ -824,8 +769,7 @@ int ssvb_barlow_bwd(const float* zi, const float* zj, int64_t n, int64_t d, int6
   // and the epilogue leaves the column partials sum_n dT, sum_n dT x~ per (row tile, warp) beside the output
   const float* inv_i = normalize ? sv.inv_i : nullptr;
   const float* inv_j = normalize ? sv.inv_j : nullptr;
-  static const bool no_fused = getenv("SSVB_BARLOW_NO_FUSED_BWD") != nullptr;  // A/B switch: dT round trip + finish kernels
-  if (!normalize && !no_fused && gemm_tma_store_allowed()) {
+  if (!normalize && gemm_tma_store_allowed()) {
     // closed-form standardisation backward inside the GEMM epilogue (see barlow_fwd_finish_kernel): the two GEMMs write
     // dzi / dzj directly (rows are 16-byte aligned: check_rows above).  normalize = 1 also needs a per-row dot with the
     // finished gradient and keeps the dT + finish-kernel path below.
@@ -872,22 +816,6 @@ int ssvb_barlow_bwd(const float* zi, const float* zj, int64_t n, int64_t d, int6
     SSVB_LAUNCH_CHECK();
   }
   const unsigned fgrid = static_cast<unsigned>(ceil_div(d, 32));
-  static const bool no_x2 = getenv("SSVB_BARLOW_NO_X2") != nullptr;  // A/B switch: one view per launch
-  if (no_x2) {
-    col_finalize_wide_kernel<<<fgrid, dim3(32, 8), 0, s>>>(part_i, nsplit, n, static_cast<int>(d), ws.colred, ws.colred + d);
-    SSVB_LAUNCH_CHECK();
-    col_finalize_wide_kernel<<<fgrid, dim3(32, 8), 0, s>>>(part_j, nsplit, n, static_cast<int>(d), ws.colred + 2 * d,
-                                                           ws.colred + 3 * d);
-    SSVB_LAUNCH_CHECK();
-    barlow_finish_kernel<<<static_cast<unsigned>(n), 256, 0, s>>>(zi, ld_zi, inv_i, sv.mean_i, sv.rstd_i, ws.dti, d, ws.colred,
-                                                                ws.colred + d, static_cast<int>(d), grad_out, dzi, ld_dzi);
-    SSVB_LAUNCH_CHECK();
-    barlow_finish_kernel<<<static_cast<unsigned>(n), 256, 0, s>>>(zj, ld_zj, inv_j, sv.mean_j, sv.rstd_j, ws.dtj, d,
-                                                                ws.colred + 2 * d, ws.colred + 3 * d, static_cast<int>(d),
-                                                                grad_out, dzj, ld_dzj);
-    SSVB_LAUNCH_CHECK();
-    return SSVB_OK;
-  }
   // both views per launch (colred = [mean dTi | sum dTi x~i | mean dTj | sum dTj x~j])
   col_finalize_wide_kernel<<<dim3(fgrid, 2), dim3(32, 8), 0, s>>>(part_i, nsplit, n, static_cast<int>(d), ws.colred,
                                                                   ws.colred + d, ws.view_stride);

@@ -552,8 +552,7 @@ static int sinkhorn_run_impl(const float* scores, int64_t b, int64_t k, int64_t 
   const bool regacc = (nwarp == 8) && (k <= static_cast<int64_t>(kSkJ) * threads);
   const bool fast = (k % 4 == 0) && (k <= 128 * kSkNV) && (ld_scores % 4 == 0) && (ld_codes % 4 == 0) &&
                     !(reinterpret_cast<uintptr_t>(scores) & 15) && !(reinterpret_cast<uintptr_t>(codes) & 15);
-  static const bool no_batch = getenv("SSVB_SK_NO_BATCH") != nullptr;  // A/B switch
-  const bool batch = fast && n_iters > 0 && nprob == kSkMaxProb && (pstride_s % 4 == 0) && (pstride_c % 4 == 0) && !no_batch;
+  const bool batch = fast && n_iters > 0 && nprob == kSkMaxProb && (pstride_s % 4 == 0) && (pstride_c % 4 == 0);
   if (batched) *batched = batch;
   if (scaling_only && !batch) return SSVB_OK;  // nothing launched: the caller falls back to sinkhorn_run
   if (nprob > 1 && !batch) {

@@ -82,7 +82,8 @@ __device__ __forceinline__ float block_reduce(float v, bool is_max, float* red) 
   return is_max ? warp_max(t) : warp_sum(t);
 }
 
-// one block per sample row r (of B'): both views' cross-entropy terms and dscores.
+// one block per sample row r (of B'): both views' cross-entropy terms and dscores.  Any K and any row alignment: the form
+// for kp8 > 4096 and for score / code rows that are not 16-byte aligned.
 __global__ void swav_ce_kernel(const float* __restrict__ scores, const float* __restrict__ codes, int64_t bp, int k,
                                int64_t ld, float inv_t, float coef /* 1/(2 B' T) */, float* __restrict__ loss_part,
                                __nv_bfloat16* __restrict__ ds, int64_t ldds) {
@@ -132,88 +133,10 @@ __global__ void swav_ce_kernel(const float* __restrict__ scores, const float* __
   }
 }
 
-// Register-cached variant (K <= 256 * EPT): every score / code row is loaded ONCE (coalesced, column = tid + e * 256) and
-// all statistics come from registers; the two maxima and the six sums are reduced together (two block reductions
-// instead of eight).  Same arithmetic as swav_ce_kernel.
-template <int EPT>
-__global__ void __launch_bounds__(256)
-swav_ce_reg_kernel(const float* __restrict__ scores, const float* __restrict__ codes, int64_t bp, int k, int64_t ld,
-                   float inv_t, float coef /* 1/(2 B' T) */, float* __restrict__ loss_part, __nv_bfloat16* __restrict__ ds,
-                   int64_t ldds) {
-  __shared__ float red[8][6];
-  const int64_t r = blockIdx.x;
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const float* s1p = scores + r * ld;
-  const float* s2p = scores + (bp + r) * ld;
-  const float* q1p = codes + r * ld;
-  const float* q2p = codes + (bp + r) * ld;
-  float t1[EPT], t2[EPT], q1[EPT], q2[EPT];
-  float m1 = -INFINITY, m2 = -INFINITY;
-#pragma unroll
-  for (int e = 0; e < EPT; ++e) {
-    const int c = threadIdx.x + e * 256;
-    const bool ok = c < k;
-    t1[e] = ok ? s1p[c] * inv_t : -INFINITY;
-    t2[e] = ok ? s2p[c] * inv_t : -INFINITY;
-    q1[e] = ok ? q1p[c] : 0.f;
-    q2[e] = ok ? q2p[c] : 0.f;
-    m1 = fmaxf(m1, t1[e]);
-    m2 = fmaxf(m2, t2[e]);
-  }
-  m1 = warp_max(m1);
-  m2 = warp_max(m2);
-  if (lane == 0) { red[w][0] = m1; red[w][1] = m2; }
-  __syncthreads();
-  m1 = red[0][0]; m2 = red[0][1];
-#pragma unroll
-  for (int i = 1; i < 8; ++i) { m1 = fmaxf(m1, red[i][0]); m2 = fmaxf(m2, red[i][1]); }
-  __syncthreads();
-  float v[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // e1, e2, a12, a21, sq1, sq2
-#pragma unroll
-  for (int e = 0; e < EPT; ++e) {
-    if (threadIdx.x + e * 256 < k) {
-      v[2] = fmaf(q1[e], t2[e], v[2]);  // sum q1 * (s2/T)
-      v[3] = fmaf(q2[e], t1[e], v[3]);
-    }
-    t1[e] = __expf(t1[e] - m1);  // exp(-inf) = 0 on the padding
-    t2[e] = __expf(t2[e] - m2);
-    v[0] += t1[e];
-    v[1] += t2[e];
-    v[4] += q1[e];
-    v[5] += q2[e];
-  }
-#pragma unroll
-  for (int i = 0; i < 6; ++i) v[i] = warp_sum(v[i]);
-  if (lane == 0) {
-#pragma unroll
-    for (int i = 0; i < 6; ++i) red[w][i] = v[i];
-  }
-  __syncthreads();
-#pragma unroll
-  for (int i = 0; i < 6; ++i) {
-    float t = 0.f;
-#pragma unroll
-    for (int ww = 0; ww < 8; ++ww) t += red[ww][i];
-    v[i] = t;
-  }
-  const float lse1 = m1 + __logf(v[0]), lse2 = m2 + __logf(v[1]);
-  if (threadIdx.x == 0) loss_part[r] = -0.5f * ((v[2] - v[4] * lse2) + (v[3] - v[5] * lse1));
-  const float i1 = v[5] / v[0], i2 = v[4] / v[1];  // softmax(s/T) * sum(q of the other view)
-  __nv_bfloat16* d1 = ds + r * ldds;
-  __nv_bfloat16* d2 = ds + (bp + r) * ldds;
-#pragma unroll
-  for (int e = 0; e < EPT; ++e) {
-    const int c = threadIdx.x + e * 256;
-    if (c < ldds) {
-      const bool ok = c < k;
-      d1[c] = __float2bfloat16_rn(ok ? -(q2[e] - t1[e] * i1) * coef : 0.f);  // d loss / d s1
-      d2[c] = __float2bfloat16_rn(ok ? -(q1[e] - t2[e] * i2) * coef : 0.f);  // d loss / d s2
-    }
-  }
-}
-
-// float4 form of the register-cached kernel (16-byte aligned rows, ld % 4 == 0, ldds % 4 == 0, ldds <= 1024 * V): thread t
-// owns columns 4 * (t + 256 * e) .. + 3 - a quarter of the load / store instructions (16-byte loads, 8-byte bf16 stores).
+// Register-cached float4 form of swav_ce_kernel (16-byte aligned rows, ld % 4 == 0, ldds % 4 == 0, ldds <= 1024 * V):
+// every score / code row is loaded ONCE and all statistics come from registers; the two maxima and the six sums are
+// reduced together (two block reductions instead of eight).  The formulas of swav_ce_kernel, summed in another order.
+// Thread t owns columns 4 * (t + 256 * e) .. + 3 (16-byte loads, 8-byte bf16 stores).
 // The padding columns [k, ld) of the score / code rows are never written by their producers: masked per element.
 template <int V>
 __global__ void __launch_bounds__(256)
@@ -537,21 +460,15 @@ int stage_ce(const float* scores, const float* codes, const SwavDims& m, int64_t
   const unsigned grid = static_cast<unsigned>(m.bp);
   const int ki = static_cast<int>(m.k);
   const float it = 1.f / temperature, coef = 0.5f / (static_cast<float>(bp_total) * temperature);
-#define SSVB_CE(E) swav_ce_reg_kernel<E><<<grid, 256, 0, s>>>(scores, codes, m.bp, ki, m.kp4, it, coef, loss_part, sv.ds, m.kp8)
 #define SSVB_CE4(V) swav_ce_reg4_kernel<V><<<grid, 256, 0, s>>>(scores, codes, m.bp, ki, m.kp4, it, coef, loss_part, sv.ds, m.kp8)
-  static const bool no_ce4 = getenv("SSVB_SWAV_NO_CE4") != nullptr;  // A/B switch
-  const bool vec = !no_ce4 && !(reinterpret_cast<uintptr_t>(scores) & 15) && !(reinterpret_cast<uintptr_t>(codes) & 15) &&
+  // the float4 kernel needs 16-byte aligned score / code rows; a ssvb_swav_dist_ce caller may pass others
+  const bool vec = !(reinterpret_cast<uintptr_t>(scores) & 15) && !(reinterpret_cast<uintptr_t>(codes) & 15) &&
                    !(reinterpret_cast<uintptr_t>(sv.ds) & 7);  // (kp4 % 4 == 0 and kp8 % 8 == 0 by construction)
   if (vec && m.kp8 <= 1 * 1024) SSVB_CE4(1);
   else if (vec && m.kp8 <= 2 * 1024) SSVB_CE4(2);
   else if (vec && m.kp8 <= 3 * 1024) SSVB_CE4(3);
   else if (vec && m.kp8 <= 4 * 1024) SSVB_CE4(4);
-  else if (m.kp8 <= 4 * 256) SSVB_CE(4);
-  else if (m.kp8 <= 8 * 256) SSVB_CE(8);
-  else if (m.kp8 <= 12 * 256) SSVB_CE(12);
-  else if (m.kp8 <= 16 * 256) SSVB_CE(16);
   else swav_ce_kernel<<<grid, 256, 0, s>>>(scores, codes, m.bp, ki, m.kp4, it, coef, loss_part, sv.ds, m.kp8);
-#undef SSVB_CE
 #undef SSVB_CE4
   SSVB_LAUNCH_CHECK();
   sum_partials_kernel<<<1, 1024, 0, s>>>(loss_part, static_cast<int>(m.bp), 1.f / static_cast<float>(bp_total), loss);
@@ -591,10 +508,9 @@ int ssvb_swav_fwd(const float* z1, const float* z2, const float* bank, const flo
   SSVB_TRY(stage_scores(z1, z2, bank, prototypes, m, ld_z1, ld_z2, ld_bank, ld_proto, sv, ws.scores, s));
   // codes per view (Sinkhorn normalises over the B' rows of ONE view)
   // the two views' code assignments (utils/losses.py:232) are independent problems of one shape: batched launches
-  static const bool no_fuse = getenv("SSVB_SWAV_NO_FUSED_CODES") != nullptr;  // A/B switch: final pass + code matrix
   const float *alpha = nullptr, *smax = nullptr;
   int kpad = 0, rc = SSVB_OK;
-  if (!no_fuse && m.kp8 <= 4 * 1024 && !(reinterpret_cast<uintptr_t>(sv.ds) & 7) &&
+  if (m.kp8 <= 4 * 1024 && !(reinterpret_cast<uintptr_t>(sv.ds) & 7) &&
       sinkhorn_scaling_only(ws.scores, m.bp, k, m.kp4, eps, n_iters, ws.sk, s, m.bp * m.kp4, &alpha, &smax, &kpad, &rc)) {
     // the iteration ran without its final pass: the cross-entropy kernel rebuilds each code row from the scaling vectors
     SSVB_TRY(rc);

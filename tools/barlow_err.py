@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Gradient / loss error of BarlowLoss against the fp64 oracle for the active code path (A/B switches come from the
-environment: SSVB_BARLOW_NO_FUSED_BWD, SSVB_BARLOW_NO_X2).  Prints one line per shape."""
+"""Gradient / loss error of BarlowLoss against the fp64 oracle for the shipped code path.  Prints one line per shape.
+The fused-vs-unfused backward error comparison of DESIGN §4.2 needs the A/B switches that commit 3683d33 still has:
+run this script at that commit to reproduce it."""
 import os
 import sys
 
