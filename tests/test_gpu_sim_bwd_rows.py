@@ -440,6 +440,42 @@ def unit_rows(x):
     return x / x.norm(dim=1, keepdim=True)
 
 
+def moco_saved_layout(n, dpad):
+    """moco.cu moco_saved: (byte offsets of qhat bf16 [npad x dpad], inv_q, inv_k, pos, lse2 [npad] fp32, pm fp32
+    [npad x dpad]; total bytes).  Carver starts every piece on a 256-byte boundary."""
+    npad = ru(n, 128)
+    offs, off = [], 0
+    for nbytes in (npad * dpad * 2, npad * 4, npad * 4, npad * 4, npad * 4, npad * dpad * 4):
+        off = ru(off, 256)
+        offs.append(off)
+        off += nbytes
+    return offs, ru(off, 256)
+
+
+def moco_finish_witness(q, kk, inv_q, inv_k, pos, lse2, acc, tau, go, n_global, normalize):
+    """moco_grad_finish_kernel restated in fp64 from the saved per-row statistics and the accumulator acc [n x d]
+    (sum_j p_aj m_j): (dq, dk, scale of dq, scale of dk), the scales being |g / |x|| before the projection."""
+    d = q.shape[1]
+    scale = go / (n_global * tau)
+    iq = inv_q.double()[:, None] if normalize else torch.ones(q.shape[0], 1, dtype=torch.float64, device=q.device)
+    ik = inv_k.double()[:, None] if normalize else torch.ones(q.shape[0], 1, dtype=torch.float64, device=q.device)
+    qh, kh = q.double() * iq, kk.double() * ik
+    # p_a0 - 1 as the kernel evaluates it: fmaf(pos, c, -lse2) and exp2 in fp32.  Near p_a0 = 1 the subtraction
+    # cancels, so one ulp of the fp32 exponent alone moves p_a0 - 1 by ~1e-5 relative (1.3e-5 at n = 200, K = 4100
+    # against an fp64 exponent; 1.2e-7 with this one)
+    c32 = (torch.tensor(LOG2E, dtype=torch.float32) / torch.tensor(tau, dtype=torch.float32)).double()
+    arg = (pos.double() * c32 - lse2.double()).float()
+    p0m1 = (torch.exp2(arg) - 1.0).double()[:, None]
+    gq = (p0m1 * kh + acc[:, :d].double()) * scale
+    gk = p0m1 * qh * scale
+    # (a row whose positive takes the whole softmax has p_a0 - 1 = 0 in fp32 and a zero dk: it must then be exactly 0)
+    den_q, den_k = (gq * iq).norm(dim=1).clamp(min=1e-30), (gk * ik).norm(dim=1).clamp(min=1e-30)
+    if normalize:
+        gq = (gq - (gq * qh).sum(1, keepdim=True) * qh) * iq
+        gk = (gk - (gk * kh).sum(1, keepdim=True) * kh) * ik
+    return gq, gk, den_q, den_k
+
+
 def run_moco(C, n, k, d, tau, zero_rows, seed):
     L = C.lib()
     g = torch.Generator().manual_seed(seed)
@@ -462,14 +498,8 @@ def run_moco(C, n, k, d, tau, zero_rows, seed):
     C.check(L.ssvb_moco_bwd(C.ptr(q), C.ptr(kk), None, C.ptr(qb), 1, n, k, d, d, d, d, 1, ctypes.c_float(tau),
                             C.ptr(gout), C.ptr(saved), C.ptr(dq), C.ptr(dk), d, d, C.ptr(ws), wsb, st), "ssvb_moco_bwd")
     torch.cuda.synchronize()
-    # moco.cu moco_saved: qhat bf16 [npad x dpad], inv_q, inv_k, pos, lse2 [npad] fp32, pm fp32 [npad x dpad]
-    npad = ru(n, 128)
-    offs, off = [], 0
-    for nbytes in (npad * dpad * 2, npad * 4, npad * 4, npad * 4, npad * 4, npad * dpad * 4):
-        off = ru(off, 256)
-        offs.append(off)
-        off += nbytes
-    assert ru(off, 256) == sb, "moco saved layout changed"
+    offs, total = moco_saved_layout(n, dpad)
+    assert total == sb, "moco saved layout changed"
     f32 = lambda i, cnt: saved[offs[i]:offs[i] + cnt * 4].view(torch.float32)
     return dict(q=q, kk=kk, qb=qb, c=LOG2E / tau, tau=tau, go=-0.8, dq=dq, dk=dk,
                 qh=saved[:n * dpad * 2].view(torch.bfloat16).view(n, dpad).float(),
@@ -489,12 +519,18 @@ def moco_witness(r, drop_tile=None):
     return c + torch.log2(lsum), p @ mb, ((p * p) @ (mb * mb).sum(1)).sqrt()
 
 
-@pytest.mark.parametrize("n,k,d,tau,zero_rows", [
+MOCO_FUSED_CASES = [
     (256, 65536, 128, 0.07, 0),   # cfg2
+    # one row block: 128 chunks, 512 partials per row, the tail loop of moco_fused_finalize_kernel (n = 128 rather than
+    # 64: over 64 rows the largest one-tile change of pm is 0.069, under 10 x MOCO_PM_TOL)
+    (128, 65536, 128, 0.07, 0),
     (200, 4100, 128, 0.07, 0),    # n not a multiple of 128, queue tail inside a tile
     (256, 4100, 64, 0.2, 37),     # zero queue rows
     (100, 16384, 128, 0.07, 5),
-])
+]
+
+
+@pytest.mark.parametrize("n,k,d,tau,zero_rows", MOCO_FUSED_CASES)
 def test_moco_fused_rows(C, n, k, d, tau, zero_rows):
     r = run_moco(C, n, k, d, tau, zero_rows, seed=n + k)
     lse_w, pm_w, rho = moco_witness(r)
@@ -512,20 +548,8 @@ def test_moco_fused_rows(C, n, k, d, tau, zero_rows):
     assert e_pm.max().item() <= MOCO_PM_TOL, f"max per-row pm error {e_pm.max().item():.3e} (row {int(e_pm.argmax())})"
     assert p_lse >= 10 * MOCO_LSE_TOL and p_pm >= 10 * MOCO_PM_TOL, f"one missing queue tile: {p_lse:.3e}, {p_pm:.3e}"
     # gradient finish (moco_grad_finish_kernel) restated from the saved blob
-    c, scale = r["c"], r["go"] / (n * r["tau"])
-    qh = r["q"].double() * r["inv_q"].double()[:, None]
-    kh = r["kk"].double() * r["inv_k"].double()[:, None]
-    # p_a0 - 1 as the kernel evaluates it: fmaf(pos, c, -lse2) and exp2 in fp32.  Near p_a0 = 1 the subtraction
-    # cancels, so one ulp of the fp32 exponent alone moves p_a0 - 1 by ~1e-5 relative (1.3e-5 at n = 200, K = 4100
-    # against an fp64 exponent; 1.2e-7 with this one)
-    c32 = (torch.tensor(LOG2E, dtype=torch.float32) / torch.tensor(r["tau"], dtype=torch.float32)).double()
-    arg = (r["pos"].double() * c32 - r["lse2"].double()).float()
-    p0m1 = (torch.exp2(arg) - 1.0).double()[:, None]
-    gq = (p0m1 * kh + r["pm"][:, :d].double()) * scale
-    gk = p0m1 * qh * scale
-    den_q, den_k = (gq * r["inv_q"].double()[:, None]).norm(dim=1), (gk * r["inv_k"].double()[:, None]).norm(dim=1)
-    gq = (gq - (gq * qh).sum(1, keepdim=True) * qh) * r["inv_q"].double()[:, None]
-    gk = (gk - (gk * kh).sum(1, keepdim=True) * kh) * r["inv_k"].double()[:, None]
+    gq, gk, den_q, den_k = moco_finish_witness(r["q"], r["kk"], r["inv_q"], r["inv_k"], r["pos"], r["lse2"], r["pm"],
+                                               r["tau"], r["go"], n, True)
     eq = ((r["dq"].double() - gq).norm(dim=1) / den_q).max().item()
     ek = ((r["dk"].double() - gk).norm(dim=1) / den_k).max().item()
     print(f"moco finish: dq {eq:.3e} dk {ek:.3e}")
