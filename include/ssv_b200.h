@@ -462,7 +462,14 @@ int ssvb_sela_self_label(const float* logits, int64_t b, int64_t k, int64_t ld, 
  *     teacher: [bs x 2 x k] contiguous, student: [bs x nv x k] contiguous, center: [k].
  *     loss = -(1/(bs nv)) sum_{b,v,k} (T_0 + T_1) log_softmax(student/temp_s),  T_g = softmax((teacher_g - center)/temp_t);
  *     gradient to the student only (the teacher runs under no_grad, models/dino.py:151-152).
- *     ssvb_dino_center_update: models/dino.py:136-141 (first != 0: center = mean of the rows).
+ *     Envelope: 1 <= k <= 65536.  k <= 8192: one CTA per sample, or (large batches) one per (sample, view) row;
+ *     8192 < k <= 65536: one thread-block cluster of ceil(k / 8192) CTAs per row, each CTA holding one 8192-column
+ *     slice, the row statistics combined through distributed shared memory.  k > 65536: SSVB_ERR_UNSUPPORTED.
+ *     The split and cluster forms use float4 accesses when k % 4 == 0 and every pointer is 16-byte aligned, scalar
+ *     accesses otherwise.
+ *     Workspace: [bs * nv] fp32 loss partials (padded to 256 bytes), then Tsum = T_0 + T_1 [bs x k] fp32.  The
+ *     backward needs it whenever bs and nv select the split form or k > 8192; the forward always.
+ *     ssvb_dino_center_update: models/dino.py:136-141 (first != 0: center = mean of the rows), any k.
  * ------------------------------------------------------------------------------------- */
 size_t ssvb_dino_workspace_bytes(int64_t bs, int64_t nv, int64_t k);
 int ssvb_dino_fwd(const float* teacher, const float* student, const float* center, int64_t bs, int64_t nv, int64_t k,

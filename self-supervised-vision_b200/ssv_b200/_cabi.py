@@ -83,7 +83,7 @@ def strerror(rc: int) -> str:
 _LIMITS = ("supported envelope (INTEGRATION.md §4): fp32 rows, row stride and feature dim multiples of 4, 16-byte aligned "
            "base pointers; d <= 256 for the similarity losses (SimclrLoss / MocoLoss / RelicLoss / PirlLoss; d <= 128 is the "
            "tuned path and the only one of the peer-memory transport); "
-           "K <= 8192 for DinoLoss")
+           "K <= 65536 for DinoLoss")
 
 
 def check(rc: int, what: str):
